@@ -7,7 +7,7 @@ its target on) through sr_run_view: stage (1) refractive tap-volume build, stage
 support-weight aggregation with fused WTA.  Metric = sum over reference views of H*W*D / time.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--workload cfg4|cfg5|cfg3|small] [--partition views|rows]
+                  [--workload cfg4|cfg5|cfg3|small] [--partition views|rows] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); reference views are dealt to ranks (north_star:
 "by reference view for multi-view runs") or, with --partition rows, every rank takes a row band of
@@ -48,6 +48,13 @@ from stereoreconstruction_b200 import scenes, sharding, types as T  # noqa: E402
 
 METRIC = "cost-volume Mpix*disp/s (build+aggregate+WTA)"
 UNIT = "Mpix*disp/s"
+# --dump-outputs: 3 float64 maps x 8 views x 2^18 pixels = 48 MiB, under the 64 MB a dump may take
+DUMP_PIXELS = 1 << 18
+
+
+def dump_pixels(h, w):
+    """The flat pixel indices --dump-outputs keeps of an h x w map: all of them, or a fixed seeded sample."""
+    return np.sort(np.random.default_rng(0).choice(h * w, min(h * w, DUMP_PIXELS), replace=False))
 
 
 def workload(name):
@@ -288,10 +295,16 @@ def main():
     ap.add_argument("--views", type=int, default=0, help="only the first N reference views (profiling aid; 0 = all)")
     ap.add_argument("--partition", default="views", choices=["views", "rows"],
                     help="multi-GPU: deal reference views to ranks (default) or give every rank a row band of every view")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what their last step returned for each reference view (depth, "
+                         "depth_index, best_cost) as DIR/<name>_view<v>.npy, float64, at a fixed seeded sample of "
+                         f"{DUMP_PIXELS} pixels per view (the whole map when it is smaller)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or (world > 1 and args.partition == "rows")):
+        raise SystemExit("--dump-outputs needs --impl ours and whole views per rank (--partition views)")
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     wl = workload(args.workload)
     w, h, V, D = wl["w"], wl["h"], wl["V"], wl["D"]
@@ -446,6 +459,12 @@ def main():
     ms_per_step, t_begin, t_end = timed_steps(my_views, args.steps, 0)
     clocks = sampler.finish(t_begin, t_end)
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs:  # before the legs below recompute (or cross-check) any view
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        pick = dump_pixels(h, w)
+        for v in my_views:
+            for name, a in (("depth", ctx.depth(v)), ("depth_index", ctx.depth_index(v)), ("best_cost", ctx.best_cost(v))):
+                np.save(os.path.join(args.dump_outputs, f"{name}_view{v}.npy"), a.reshape(-1)[pick].astype(np.float64))
     # per-stage device times: one more step with the library's per-stage events on (which serialises the
     # views on the context stream: a kernel's duration is then its own, not stretched by the overlap)
     ctx.set_profiling(True)

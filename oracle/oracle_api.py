@@ -49,7 +49,7 @@ def _cpu_stamp():
 
 
 def build(verbose=False):
-    """Compile the oracle (and oracle/_ref when /root/reference exists).  -march=native is used,
+    """Compile the oracle (and oracle/_ref when REF names the reference's source tree, see Makefile).  -march=native is used,
     so the library is rebuilt when the host CPU differs from the one it was built on."""
     os.makedirs(os.path.join(_HERE, "_build"), exist_ok=True)
     stamp = os.path.join(_HERE, "_build", "cpu.stamp")
@@ -85,7 +85,7 @@ def lib():
 
 
 def ref_lib():
-    """The reference's own leaf sources compiled from /root/reference (oracle/_ref/libref.so), or
+    """The reference's own sources compiled from its source tree (oracle/_ref/libref.so), or
     None when neither the reference tree nor a prebuilt library is available."""
     global _REF
     if _REF is None:

@@ -1,11 +1,11 @@
 #!/usr/bin/env python
 """Derives the small `bunny` fixture of tests/golden/bunny/ from the reference's example data.
 
-  python tests/golden/make_bunny.py      (build container only: reads /root/reference/example)
+  REF=<reference source tree> python tests/golden/make_bunny.py      (reads $REF/example)
 
 BASELINE.json configs[0] and [1] are the reference's `example/project.xml` 'bunny' image set (8
 calibrated, lens-distorted cameras, 1024x768 RGBA PNGs whose alpha channel is the object mask).
-The GPU box has no /root/reference, and 11 MB of PNGs do not belong in the history, so the
+The tests must run without the reference's sources, and 11 MB of PNGs do not belong in the history, so the
 fixture is: the 8 camera entries of the XML verbatim as JSON (projection matrix + distortion),
 and the images reduced to 1/4 size (256x192, PIL LANCZOS on RGB, alpha thresholded so the mask
 stays binary).  Both the oracle and the GPU path read these identically pre-scaled images with
@@ -18,7 +18,7 @@ import re
 import numpy as np
 from PIL import Image
 
-REF = "/root/reference/example"
+REF = os.path.join(os.environ.get("REF", ""), "example")
 HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "bunny")
 SCALE = 0.25
 

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Full-size (1024 x 768) `bunny` golden vectors from THE REFERENCE ITSELF (BASELINE configs[0], [1]).
 
-  python tests/golden/make_bunny_full.py     (build container only: reads /root/reference/example and
-                                              needs oracle/_ref = the reference compiled where it lies)
+  REF=<reference source tree> python tests/golden/make_bunny_full.py     (reads $REF/example and needs
+                                              oracle/_ref = the reference compiled where it lies)
 
 The reference's own example data at its own size: real calibrated, lens-distorted cameras, real object
 masks, flat regions.  11 MB of PNGs do not belong in the history and the reference needs minutes per full
@@ -40,7 +40,7 @@ from oracle import oracle_api as O  # noqa: E402
 from stereoreconstruction_b200 import types as T  # noqa: E402
 import golden_cases as G  # noqa: E402
 
-REF = "/root/reference/example"
+REF = os.path.join(os.environ.get("REF", ""), "example")
 OUT = os.path.join(HERE, "bunny_full")
 MIN_D, MAX_D, LEVELS = 30.0, 55.0, 100     # brackets the object for the cameras of example/project.xml (golden_cases.py)
 MVS_REF, BAND = 2, (396, 428)              # 32 rows through the middle of the object

@@ -1,12 +1,12 @@
 #!/usr/bin/env python
 """Generates the committed golden fixtures of tests/golden/.
 
-  python tests/golden/make_golden.py        (run in the build container, where /root/reference exists)
+  REF=<reference source tree> python tests/golden/make_golden.py     (builds oracle/_ref from that tree first)
 
 ref_leaves.npz    outputs of the REFERENCE'S OWN sources (util/lineiter.cpp, util/ray.cpp,
                   util/vectorimage.cpp, stereo/adaptiveweight.cpp, stereo/geodesicweight.cpp,
                   project/camera.cpp compiled where they lie into oracle/_ref/libref.so) on seeded inputs.  They pin the oracle
-                  — and through it the CUDA path — on machines where /root/reference is absent.
+                  — and through it the CUDA path — on machines without the reference's sources.
 ref_mvs.npz       END-TO-END outputs of the reference's own MultiViewStereo class (stereo/multiviewstereo.cpp
                   + project/camera.cpp + the leaves, compiled where they lie, driven initialize() ->
                   runTask() by oracle/ref_glue_mvs.cpp): neighbour lists, depths before and after the
@@ -47,7 +47,7 @@ def _dp(a):
 def ref_leaves():
     REF = O.ref_lib()
     if REF is None:
-        raise SystemExit("oracle/_ref/libref.so is not built: run `make -C oracle` where /root/reference exists")
+        raise SystemExit("oracle/_ref/libref.so is not built: run `make -C oracle REF=<reference source tree>`")
     out = {}
     # --- LineIterator / clipLine (util/lineiter.hpp:32-118, util/lineiter.cpp:44-88)
     cases, w, h = G.line_cases()

@@ -239,33 +239,53 @@ def _with_model(cams, model):
     return out
 
 
-def test_host_camera_class_matches_reference_camera(tmp_path):
-    """CPU: the C++ `Project` + `Camera` classes of include/ (XML -> Camera::setP -> updateOthers -> toPod) on
-    the 8 cameras of the reference's example/project.xml (tests/golden/bunny/cameras.json) and on refractive
-    arc cameras, against the REFERENCE'S OWN Camera::setP / set (project/camera.cpp compiled where it lies,
-    oracle/_ref): K, R, t, C, the principal ray and the inverses agree to rounding."""
+def bunny_cameras():
+    """The 8 cameras of the reference's example/project.xml (tests/golden/bunny/cameras.json)."""
     import json
-    from oracle import oracle_api as O
-    REF = O.ref_lib()
-    if REF is None:
-        pytest.skip("oracle/_ref/libref.so not available")
     from bunny_util import DIR
     meta = json.load(open(os.path.join(DIR, "cameras.json")))
-    cams = [T.camera_from_P(c["P"], dist=c["dist"]) for c in meta["cameras"]]
+    return [T.camera_from_P(c["P"], dist=c["dist"]) for c in meta["cameras"]]
+
+
+def projection_matrices(cams):
+    """What write_project puts into the XML for each camera."""
+    out = []
+    for c in cams:
+        K, R, t = (np.array(getattr(c, f)[:]) for f in ("K", "R", "t"))
+        out.append(K.reshape(3, 3) @ np.hstack([R.reshape(3, 3), t[:, None]]))
+    return out
+
+
+def test_host_camera_class_matches_reference_camera(tmp_path):
+    """CPU: the C++ `Project` + `Camera` classes of include/ (XML -> Camera::setP -> updateOthers -> toPod) on
+    the 8 cameras of the reference's example/project.xml (tests/golden/bunny/cameras.json), against the
+    REFERENCE'S OWN Camera::setP (project/camera.cpp compiled where it lies, oracle/_ref): K, R, t, C, the
+    principal ray and the inverses agree to rounding.  Where oracle/_ref is not built, the comparison is with
+    tests/golden/ref_pins/host_cameras.npz, which holds this C++ Camera class's own output from when it agreed
+    with the reference (tests/golden/make_ref_pins.py): a regression pin, not an independent check."""
+    from oracle import oracle_api as O
+    REF = O.ref_lib()
+    cams = bunny_cameras()
+    n = C.sizeof(T.SrCamera)
+    if REF is not None:
+        refs = []
+        for P in projection_matrices(cams):
+            ref = O.OrcCamera()
+            REF.ref_camera_from_P(np.ascontiguousarray(P).ctypes.data_as(C.POINTER(C.c_double)), C.byref(ref))
+            refs.append(ref)
+    else:
+        buf = np.load(os.path.join(ROOT, "tests", "golden", "ref_pins", "host_cameras.npz"))["cams"].tobytes()
+        refs = [O.OrcCamera.from_buffer_copy(buf[i * n:(i + 1) * n]) for i in range(len(buf) // n)]
+    assert len(refs) == len(cams)
     h, w = 8, 8
     blank = [np.zeros((h, w, 4), np.uint8)] * len(cams)
     xml = write_project(str(tmp_path), cams, blank, [np.full((h, w), 255, np.uint8)] * len(cams))
     r = subprocess.run([HARNESS, "--cameras", xml, str(tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
     raw = open(os.path.join(str(tmp_path), "cams.bin"), "rb").read()
-    n = C.sizeof(T.SrCamera)
     assert len(raw) == n * len(cams)
-    for i, c in enumerate(cams):
+    for i, (c, ref) in enumerate(zip(cams, refs)):
         host = T.SrCamera.from_buffer_copy(raw[i * n:(i + 1) * n])
-        K, R, t = (np.array(getattr(c, f)[:]) for f in ("K", "R", "t"))
-        P = K.reshape(3, 3) @ np.hstack([R.reshape(3, 3), t[:, None]])  # what write_project put into the XML
-        ref = O.OrcCamera()
-        REF.ref_camera_from_P(np.ascontiguousarray(P).ctypes.data_as(C.POINTER(C.c_double)), C.byref(ref))
         for f in ("K", "Kinv", "R", "Rinv", "t", "C", "prin_dir"):
             a, b = np.array(getattr(host, f)[:]), np.array(getattr(ref, f)[:])
             assert np.allclose(a, b, rtol=1e-9, atol=1e-9), (i, f, np.abs(a - b).max())
