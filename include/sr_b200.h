@@ -126,8 +126,7 @@ int sr_get_stage_ms(sr_ctx *ctx, double *out4);
  * FP32, [2] labels forced to FP64, [3] FP64 verifications, [4] pixels evaluated in FP64 only,
  * [5] bit pattern (low 32 bits, IEEE float) of the largest |ncc32 - ncc64| seen on a verified label,
  * [6] verified labels whose FP32 value lay outside its error bar (must be 0),
- * [7] labels dropped by the subset bound of the two-level sweep whose full FP32 evaluation would have
- * made them candidates (must be 0; with the switch on every dropped label is also evaluated in full). */
+ * [7] reserved, always 0. */
 int sr_get_match_stats(sr_ctx *ctx, uint64_t *out8);
 /* Self-check counters of the refractive tap-volume build (same switch, SR_MATCH_STATS=1): with
  * the switch on, every interpolated label is ALSO projected exactly.  out4[0] labels taken from

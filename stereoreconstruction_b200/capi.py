@@ -138,6 +138,8 @@ class Context:
         return dict(interpolated=int(out[0]), guard_fallbacks=int(out[1]), tap_mismatches=int(out[2]))
 
     def match_stats(self):
+        """Counters of sr_get_match_stats.  prescreen_false_drops is slot 7, reserved and always 0 since the
+        subset-bound sweep it counted was removed; the key stays so that callers reading it keep working."""
         out = np.zeros(8, np.uint64)
         self._ck(self._L.sr_get_match_stats(self._h, _p(out)))
         return dict(pixels=int(out[0]), screened=int(out[1]), forced=int(out[2]), verified=int(out[3]),

@@ -15,7 +15,6 @@
 #include "sr_match_dispatch.cuh"
 #include "sr_build_refr.cuh"
 #include "sr_curve.cuh"
-#include "sr_pipeline.cuh"
 
 using namespace sr;
 
@@ -147,13 +146,6 @@ struct sr_ctx {
     // stream: sr_get_depth(v) overlaps the views enqueued after v instead of joining all of them.
     std::vector<cudaEvent_t> view_done;
     cudaStream_t copy_stream = nullptr;
-    bool use_pipeline = false;  // SR_PIPELINE=1: build and screen as roles of ONE launch (sr_pipeline.cuh; measured slower: DESIGN.md)
-    int pipe_lag = 128;        // tiles between a tile's build and its screen (SR_PIPE_LAG)
-    size_t pipe_ring_bytes = (size_t)1 << 30;  // tap ring of the pipeline kernel (SR_PIPE_RING_MB)
-    int32_t *d_ring = nullptr;
-    size_t ring_cap = 0;
-    int *d_pipe_flags = nullptr;  // built[ntiles], done[ntiles], ticket
-    size_t pipe_flags_cap = 0;
     ncclComm_t comm = nullptr;
     int rank = 0, nranks = 1;
     // per-stage CUDA-event timing (sr_set_profiling): [begin, after build, after match] per band
@@ -322,7 +314,6 @@ int sr_ctx_create(int device, sr_ctx **out) {
     if (const char *mb = getenv("SR_TAP_BUDGET_MB")) c->tap_budget = (size_t)atoll(mb) << 20;
     if (const char *sc = getenv("SR_MATCH_SCREEN")) c->use_screen = atoi(sc) != 0;
     if (const char *sb = getenv("SR_BUILD_REFR")) c->use_refr_build = atoi(sb) != 0;
-    if (const char *sp = getenv("SR_PIPELINE")) c->use_pipeline = atoi(sp) != 0;
     if (const char *sn = getenv("SR_LANES")) c->num_lanes = std::min((int)sr_ctx::MAX_LANES, std::max(1, atoi(sn)));
     if (c->num_lanes > 1) {
         bool ok = cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) == cudaSuccess;
@@ -332,8 +323,6 @@ int sr_ctx_create(int device, sr_ctx **out) {
         ok = ok && cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) == cudaSuccess;
         if (!ok) c->num_lanes = 1;
     }
-    if (const char *sl = getenv("SR_PIPE_LAG")) c->pipe_lag = std::max(1, atoi(sl));
-    if (const char *sr_ = getenv("SR_PIPE_RING_MB")) c->pipe_ring_bytes = (size_t)std::max(1, atoi(sr_)) << 20;
     if (const char *sk = getenv("SR_BUILD_CHUNK")) c->refr_chunk = std::max(4, atoi(sk));
     if (const char *ss = getenv("SR_MATCH_STATS")) {
         if (atoi(ss) != 0 && cudaMalloc(&c->d_stats, 16 * sizeof(unsigned long long)) == cudaSuccess)
@@ -357,8 +346,6 @@ void sr_ctx_destroy(sr_ctx *c) {
     dfree(c->d_volume);
     dfree(c->d_peaks);
     dfree(c->d_stats);
-    dfree(c->d_ring);
-    dfree(c->d_pipe_flags);
     for (sr_ctx::Lane &L : c->lanes) {
         if (L.stream) cudaStreamSynchronize(L.stream);
         dfree(L.d_rays);
@@ -539,130 +526,6 @@ static int init_peaks(sr_ctx *ctx, int ref) {
     return SR_OK;
 }
 
-// sr_pipeline.cuh: support weights, then tap build + screen + verify + WTA of rows [r0, r1) as one launch.
-static int run_view_pipeline(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn, int r0, int r1) {
-    const sr_params &P = ctx->params;
-    cudaStream_t st = ctx->stream;
-    const int w = ctx->w, h = ctx->h, D = P.num_levels, rows = r1 - r0;
-    ViewDev &A = ctx->views[ref];
-    int rc = init_peaks(ctx, ref);
-    if (rc) return rc;
-    ctx->vol_elems = 0;
-    if (ctx->cancel.load()) return fail(ctx, SR_ERR_CANCELLED, "cancelled");
-    const size_t wn = (size_t)(2 * P.radius + 1) * (2 * P.radius + 1);
-    const size_t plane = (size_t)rows * w;
-    const size_t need_w = wn * plane * 8;
-    if (need_w > ctx->weights_cap) {
-        CK(cudaStreamSynchronize(st));
-        dfree(ctx->d_weights);
-        ctx->weights_cap = 0;
-        CK(cudaMalloc(&ctx->d_weights, need_w));
-        ctx->weights_cap = need_w;
-    }
-    const int tiles_x = (w + 31) / 32, tiles_y = (rows + SCREEN2_TILE_ROWS - 1) / SCREEN2_TILE_ROWS;
-    const int ntiles = tiles_x * tiles_y;
-    const size_t tile_bytes = (size_t)nn * SCREEN2_TILE_ROWS * D * 32 * 4;
-    const int lag = std::min(ctx->pipe_lag, std::max(1, ntiles));
-    // the ring must be longer than the lag (a build block may only wait for an older screen block)
-    const int ring_tiles = (int)std::min<size_t>((size_t)ntiles, std::max<size_t>((size_t)lag + 64, ctx->pipe_ring_bytes / tile_bytes));
-    const size_t need_ring = (size_t)ring_tiles * tile_bytes;
-    if (need_ring > ctx->ring_cap) {
-        CK(cudaStreamSynchronize(st));
-        dfree(ctx->d_ring);
-        ctx->ring_cap = 0;
-        CK(cudaMalloc(&ctx->d_ring, need_ring));
-        ctx->ring_cap = need_ring;
-    }
-    const size_t need_flags = ((size_t)2 * ntiles + 1) * sizeof(int);
-    if (need_flags > ctx->pipe_flags_cap) {
-        CK(cudaStreamSynchronize(st));
-        dfree(ctx->d_pipe_flags);
-        ctx->pipe_flags_cap = 0;
-        CK(cudaMalloc(&ctx->d_pipe_flags, need_flags));
-        ctx->pipe_flags_cap = need_flags;
-    }
-    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
-    if (ctx->profiling) {
-        for (int k = 0; k < 3; ++k) CK(cudaEventCreate(&ev[k]));
-        CK(cudaEventRecord(ev[0], st));
-        CK(cudaEventRecord(ev[1], st));  // (no separate build stage)
-    }
-    CK(cudaMemsetAsync(ctx->d_pipe_flags, 0, need_flags, st));
-    {
-        WeightArgs wa;
-        memset(&wa, 0, sizeof(wa));
-        wa.rgba = A.rgba;
-        wa.mask = A.mask;
-        wa.edges = A.edges;
-        wa.W = ctx->d_weights;
-        wa.w = w;
-        wa.h = h;
-        wa.row0 = r0;
-        wa.rows = rows;
-        wa.radius = P.radius;
-        const unsigned gx = (unsigned)((plane + 127) / 128);
-        if (P.weight_kind == SR_WEIGHT_ADAPTIVE)
-            weights_adaptive_kernel<<<gx, 128, (P.radius + 1) * sizeof(double), st>>>(wa);
-        else
-            launch_geodesic(wa, gx, st);
-        CKL();
-    }
-    PipeArgs pa;
-    memset(&pa, 0, sizeof(pa));
-    MatchArgs &ma = pa.m;
-    ma.W = ctx->d_weights;
-    ma.maskL = A.mask;
-    ma.grayL = A.gray_pix;
-    for (int j = 0; j < nn; ++j) {
-        const ViewDev &B = ctx->views[nbrs[j]];
-        ma.grayR[j] = B.gray_pix;
-        ma.grayRf[j] = B.gray_pix_f;
-        PipeNbr &nb = pa.nb[j];
-        nb.cam = ctx->cams[nbrs[j]];
-        refr_pixel_map(nb.cam, true, P.image_scale, nb.Kn, nb.fxs, nb.cxs, nb.fys, nb.cys);
-        nb.mask = B.all_white ? nullptr : B.mask;
-    }
-    ma.pitch_f = screen_pitch(w);
-    ma.depth_table = ctx->d_depth_table;
-    ma.out_index = A.index;
-    ma.out_depth = A.depth;
-    ma.out_best = A.best;
-    ma.w = w;
-    ma.h = h;
-    ma.win_w = std::max(0, w - 2 * P.radius);
-    ma.win_h = std::max(0, h - 2 * P.radius);
-    ma.row0 = r0;
-    ma.rows = rows;
-    ma.D = D;
-    ma.num_nbrs = nn;
-    ma.select_kind = P.select_kind;
-    ma.depth_up = (P.max_depth >= P.min_depth) ? 1 : 0;
-    ma.use_screen = 1;
-    ma.stats = ctx->d_stats;
-    ma.second_best_factor = P.second_best_factor;
-    ma.ncc_threshold = P.ncc_threshold;
-    memcpy(pa.prin, ctx->cams[ref].prin_dir, sizeof(pa.prin));
-    memcpy(pa.C, ctx->cams[ref].C, sizeof(pa.C));
-    pa.rays = ctx->d_rays;
-    pa.ring = ctx->d_ring;
-    pa.built = ctx->d_pipe_flags;
-    pa.done = ctx->d_pipe_flags + ntiles;
-    pa.ticket = reinterpret_cast<unsigned *>(ctx->d_pipe_flags + 2 * (size_t)ntiles);
-    pa.tiles_x = tiles_x;
-    pa.ntiles = ntiles;
-    pa.ring_tiles = ring_tiles;
-    pa.lag = lag;
-    pa.check = ctx->d_stats ? ctx->d_stats + 8 : nullptr;
-    cudaError_t e = launch_pipeline(P.radius, pa, st);
-    ++ctx->launches;
-    if (e != cudaSuccess) return fail(ctx, SR_ERR_CUDA, std::string("pipeline kernel: ") + cudaGetErrorString(e));
-    if (ctx->profiling) {
-        CK(cudaEventRecord(ev[2], st));
-        for (int k = 0; k < 3; ++k) ctx->prof_events.push_back(ev[k]);
-    }
-    return SR_OK;
-}
-
 int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     int rc = check_view(ctx, ref);
     if (rc) return rc;
@@ -683,19 +546,6 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     if (r0 >= r1) return fail(ctx, SR_ERR_INVALID, "empty row range");
     const size_t n = (size_t)w * h;
     ViewDev &A = ctx->views[ref];
-
-    {   // MultiViewStereo label path with refractive neighbours: build and screen as one launch
-        bool pipe = ctx->use_pipeline && ctx->use_screen && ctx->use_refr_build && P.select_kind == SR_SELECT_MVS &&
-                    P.cost_kind == SR_COST_NCC_MVS && !P.keep_cost_volume && pipeline_supported(P.radius);
-        for (int j = 0; j < nn; ++j) pipe = pipe && ctx->cams[nbrs[j]].is_refractive;
-        if (pipe) {
-            JOIN();
-            rays_kernel<<<(unsigned)(((size_t)(r1 - r0) * w + 127) / 128), 128, 0, ctx->stream>>>(ctx->cams[ref], w, h, r0, r1 - r0,
-                                                                                                   P.image_scale, ctx->d_rays);
-            CKL();
-            return run_view_pipeline(ctx, ref, nbrs, nn, r0, r1);
-        }
-    }
 
     // Where this view runs: one of the two lanes (its own stream and scratch), or the context stream when
     // something context-wide is written (kept volume, peak lists, statistics, per-stage timing).

@@ -8,10 +8,6 @@
 
 namespace sr {
 
-#ifndef SR_SCREEN2
-#define SR_SCREEN2 1  // 0: A/B against the round-1 screen kernel for r <= 2
-#endif
-
 template <int R> struct LanesFor { static constexpr int G = (R <= 2) ? 1 : (R == 3) ? 2 : (R <= 5) ? 4 : (R <= 7) ? 8 : (R <= 10) ? 16 : 32; };
 
 // Radii with a compiled match kernel.  SR_FEW_RADII (the default build, capi.py) leaves out 6-12 to
@@ -43,35 +39,21 @@ cudaError_t launch_match_rc(const MatchArgs &a, cudaStream_t st) {
 template <int R>
 cudaError_t launch_match_screen(const MatchArgs &a, cudaStream_t st) {
     constexpr int G = LanesFor<R>::G;  // (two lanes per pixel at r = 2 measured 1.7x slower: 35.8 vs 20.4 ms)
-    constexpr int PPB = SCREEN_BLOCK / G;
-    const size_t npix = (size_t)a.rows * a.w;
-    const unsigned grid = (unsigned)((npix + PPB - 1) / PPB);
-#if SR_SCREEN2
-    if (G == 1) {  // thread-per-pixel radii: sr_screen2.cuh (one warp per block)
-        constexpr int R2 = (G == 1) ? R : 1;
-        if (a.stats) return launch_screen2<R2, true, 0>(a, st);
+    if constexpr (G == 1) {  // thread-per-pixel radii: sr_screen2.cuh, the row pitch a compile-time constant
+        if (a.stats) return launch_screen2<R, true, 0>(a, st);
         switch (a.pitch_f) {
-            case 1024: return launch_screen2<R2, false, 1024>(a, st);
-            case 2048: return launch_screen2<R2, false, 2048>(a, st);
-            case 4096: return launch_screen2<R2, false, 4096>(a, st);
-            default: return launch_screen2<R2, false, 0>(a, st);
+            case 1024: return launch_screen2<R, false, 1024>(a, st);
+            case 2048: return launch_screen2<R, false, 2048>(a, st);
+            case 4096: return launch_screen2<R, false, 4096>(a, st);
+            default: return launch_screen2<R, false, 0>(a, st);
         }
+    } else {  // lane groups: sr_match_screen.cuh, one warp per block
+        constexpr int PPB = SCREEN_BLOCK / G;
+        const unsigned grid = (unsigned)(((size_t)a.rows * a.w + PPB - 1) / PPB);
+        if (a.stats) match_mvs_screen_kernel<R, G, true><<<grid, SCREEN_BLOCK, 0, st>>>(a);
+        else match_mvs_screen_kernel<R, G, false><<<grid, SCREEN_BLOCK, 0, st>>>(a);
         return cudaGetLastError();
     }
-#endif
-    if (a.stats) {
-        match_mvs_screen_kernel<R, G, true, 0><<<grid, SCREEN_BLOCK, 0, st>>>(a);
-    } else if (G == 1) {  // thread-per-pixel radii: the row pitch is a compile-time constant
-        switch (a.pitch_f) {
-            case 1024: match_mvs_screen_kernel<R, G, false, (G == 1) ? 1024 : 0><<<grid, SCREEN_BLOCK, 0, st>>>(a); break;
-            case 2048: match_mvs_screen_kernel<R, G, false, (G == 1) ? 2048 : 0><<<grid, SCREEN_BLOCK, 0, st>>>(a); break;
-            case 4096: match_mvs_screen_kernel<R, G, false, (G == 1) ? 4096 : 0><<<grid, SCREEN_BLOCK, 0, st>>>(a); break;
-            default: match_mvs_screen_kernel<R, G, false, 0><<<grid, SCREEN_BLOCK, 0, st>>>(a); break;
-        }
-    } else {
-        match_mvs_screen_kernel<R, G, false, 0><<<grid, SCREEN_BLOCK, 0, st>>>(a);
-    }
-    return cudaGetLastError();
 }
 
 template <int R>

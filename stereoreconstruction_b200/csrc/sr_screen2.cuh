@@ -41,43 +41,12 @@
 
 namespace sr {
 
-#ifndef SR_SCREEN2_ABL
-#define SR_SCREEN2_ABL 0  // 1-4: timing ablations of the label loop (wrong results; profiling only)
-#endif
-#ifndef SR_SCREEN2_STAGE
-#define SR_SCREEN2_STAGE 0  // 1: the chunk's neighbour band staged in shared memory by bulk async copies (TMA engine), windows by LDS
-#endif
-#ifndef SR_SCREEN2_LV
-#define SR_SCREEN2_LV 1  // NL = 2: FFMA2 vectorised across the two labels (scalar weight operand) instead of two taps
-#endif
-#ifndef SR_SCREEN2_PRE
-#define SR_SCREEN2_PRE 0  // 1: two-level sweep (subset bound first, full window for the survivors)
-#endif
-#ifndef SR_SCREEN2_SWP
-#define SR_SCREEN2_SWP 0  // 1: software-pipelined label loop (next label's window loads ride with this label's FFMA2s)
-#endif
-#ifndef SR_SCREEN2_NACC
-#define SR_SCREEN2_NACC 1  // accumulator pairs per window sum (one-pass form)
-#endif
-#ifndef SR_SCREEN2_NL
-#define SR_SCREEN2_NL 2  // labels evaluated together per loop iteration (independent chains: ILP within the warp)
-#endif
-#ifndef SR_SCREEN2_ONEPASS
-#define SR_SCREEN2_ONEPASS 1  // 0: A/B against the two-pass (mean first) form of the screen
-#endif
-constexpr float SCREEN_CORR_MAX = 100.0f;  // two-pass form: n_inactive * meanR^2 <= this * s3, else FP64 decides
-constexpr float SCREEN_EPS_MAX = 5e-3f;    // one-pass form: a wider error bar means FP64 decides
-constexpr float SCREEN_SKIP = -2.0f;       // "no value": below every possible lower bound
+constexpr float SCREEN_EPS_MAX = 5e-3f;  // a wider error bar means FP64 decides
+constexpr float SCREEN_SKIP = -2.0f;     // "no value": below every possible lower bound
 
 // Shared memory of one screening warp.
-constexpr int STAGE_BW = 64, STAGE_BH = 16;  // staged band: floats per row (multiple of 4), rows
 template <bool STATS>
 struct alignas(16) Screen2Smem {
-#if SR_SCREEN2_STAGE
-    float box[STAGE_BH][STAGE_BW];       // rows [y0, y0 + bh) x columns [x0, x0 + bw) of the neighbour's FP32 plane
-    unsigned long long mbar;             // completion barrier of the bulk copies
-    unsigned long long pad_;
-#endif
     int32_t tap_ring[2][TAP_CHUNK][32];
     float ub_ring[TAP_CHUNK][32];    // ncc32 + eps of the chunk's labels (SCREEN_FORCE: FP64 decides)
     int32_t q_lab[SCREEN_QCAP][32];  // (neighbour << 16) | label
@@ -92,16 +61,16 @@ struct alignas(16) Screen2Smem {
     int st_verified[STATS ? 32 : 1], st_viol[STATS ? 32 : 1];
 };
 
-// Register slot i of the window arrays holds window tap k = screen2_slot_tap<R>(i) (row-major k).  For the
-// 5x5 window the first PRE_TAPS slots are the taps of the pre-screen (the centre 3x3 block and the tap left
-// of it), so that they form whole FFMA2 pairs.
-constexpr int SCREEN2_PRE_TAPS = 10;
+// Register slot i of the window arrays holds window tap k = screen2_slot_tap<R>(i) (row-major k).  The
+// 5x5 window starts with the centre 3x3 block and the tap left of it, then the rest in row-major order.
+// The slot order is the order in which the FP32 window sums accumulate, so it fixes the screened values to
+// the last bit (and the error bars were checked with it): keep it.
 template <int R>
 __host__ __device__ constexpr int screen2_slot_tap(int i) {
     if (R != 2) return i;
-    constexpr int pre[SCREEN2_PRE_TAPS] = {6, 7, 8, 11, 12, 13, 16, 17, 18, 10};
+    constexpr int centre[10] = {6, 7, 8, 11, 12, 13, 16, 17, 18, 10};
     constexpr int rest[15] = {0, 1, 2, 3, 4, 5, 9, 14, 15, 19, 20, 21, 22, 23, 24};
-    return i < SCREEN2_PRE_TAPS ? pre[i] : rest[i - SCREEN2_PRE_TAPS];
+    return i < 10 ? centre[i] : rest[i - 10];
 }
 
 __device__ __forceinline__ int32_t lds_b32(unsigned addr) {
@@ -110,33 +79,6 @@ __device__ __forceinline__ int32_t lds_b32(unsigned addr) {
     return v;
 }
 __device__ __forceinline__ void sts_f32(unsigned addr, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v)); }
-
-// Bulk asynchronous copy (TMA engine, no tensor map: one contiguous run of bytes) and its mbarrier.
-__device__ __forceinline__ void mbar_init(unsigned mbar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mbar), "r"(count));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned mbar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned mbar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(mbar)
-                 : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned mbar, unsigned parity) {
-    unsigned ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok)
-                 : "r"(mbar), "r"(parity)
-                 : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ float lds_f32(unsigned addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
 
 // ---- the rare paths: free functions with by-value arguments, so that the screening warp's register
 // arrays (weights, dl) never have to be addressable ------------------------------------------------
@@ -309,27 +251,20 @@ __device__ __noinline__ Screen2Cold screen2_process_pending(const MatchArgs &a, 
     return r;
 }
 
-// One screening warp: 32 consecutive pixels of the band, one per lane.
+// One screening warp: 32 consecutive pixels of the band, one per lane.  PITCH: compile-time row pitch of
+// the FP32 gray planes (0: run-time a.pitch_f).
 template <int R, bool STATS, int PITCH>
 struct Screener {
     static constexpr int WS = 2 * R + 1, WN = WS * WS;
     static constexpr unsigned FULL = 0xffffffffu;
-    static constexpr bool ONEPASS = SR_SCREEN2_ONEPASS != 0;
 
     const MatchArgs &a;
     Screen2Smem<STATS> &sm;
     const int lane;
-    // wtf: support weights; c1f: one-pass dl_i w_i / sqrt(s2), two-pass dl_i / sqrt(s2)
+    // wtf: support weights w_i; c1f: dl_i w_i / sqrt(s2)
     float wtf[WN], c1f[WN];
-    // one-pass: k0 = 2 totW - n_a, k1 = SDL / sqrt(s2), error bar e0 + e1 * kappa
-    // two-pass: k0 = n_inactive, e0 = the pixel's error-bar class
+    // k0 = 2 totW - n_a, k1 = SDL / sqrt(s2), error bar e0 + e1 * kappa
     float inv_totWf, k0, k1, e0, e1, lower32;
-    float pre_sdl_n, pre_inv_n, pre_E;  // pre-screen: sum_A dl / n_A, 1 / n_A, centred energy of dl on A
-    int n_prerej, n_prebad;              // STATS only
-    // SR_SCREEN2_STAGE: the staged band of this chunk (warp-uniform)
-    unsigned box_addr, stage_phase;
-    int box_x0, box_y0;
-    bool use_box;
     int qn, my_win_w, first_pid;
     unsigned pend;
     bool alive;
@@ -391,29 +326,11 @@ struct Screener {
         for (int i = 0; i < WN; ++i) {
             const int k = screen2_slot_tap<R>(i);
             wtf[i] = (float)wt[k];
-            c1f[i] = ONEPASS ? (float)((gl[k] * rs2) * wt[k]) : (float)(gl[k] * rs2);
+            c1f[i] = (float)((gl[k] * rs2) * wt[k]);
         }
         const bool has_inactive = ninact != 0;
-        {   // pre-screen subset A = slots [0, SCREEN2_PRE_TAPS): active taps only (dl = 0 on the others)
-            double nA = 0.0, sA = 0.0, qA = 0.0;
-#pragma unroll
-            for (int i = 0; i < (R == 2 ? SCREEN2_PRE_TAPS : 0); ++i) {
-                const int k = screen2_slot_tap<R>(i);
-                if (wt[k] > 0.0) {
-                    const double d = gl[k] * rs2;
-                    nA += 1.0;
-                    sA += d;
-                    qA += d * d;
-                }
-            }
-            const double EA = (nA >= 2.0) ? qA - sA * sA / nA : 0.0;
-            pre_sdl_n = (nA > 0.0) ? (float)(sA / nA) : 0.0f;
-            pre_inv_n = (nA > 0.0) ? (float)(1.0 / nA) : 0.0f;
-            pre_E = (float)(EA * (1.0 - 1e-6));  // (rounded down: a smaller energy only weakens the bound)
-            if (!(pre_E > 0.0f) || all_slow) pre_E = 0.0f;
-        }
         inv_totWf = (float)(1.0 / totW);
-        if (ONEPASS) {
+        {
             const double na = (double)(WN - ninact);
             const double sigma = fabs(SDL * rs2) * sqrt(na) / totW;
             const double u = 5.9604644775390625e-8;  // 2^-24
@@ -422,11 +339,6 @@ struct Screener {
             e0 = (float)(1.5 * u * (6.0 + 7.5 * sigma) + 3e-7);
             e1 = (float)(1.5 * u * (29.0 + 7.5 * sigma));
             if (!(e1 < 1.0f)) e1 = 1.0f;  // (all_slow pixels: unused)
-        } else {
-            k0 = (float)ninact;
-            k1 = 0.0f;
-            e0 = (s2 >= 100.0 * WN && !has_inactive) ? SCREEN_EPS_TIGHT : SCREEN_EPS_LOOSE;
-            e1 = 0.0f;
         }
         // lanes that screen nothing (no pixel, or an ill-conditioned reference window that only the exact
         // filter may judge) see an empty interior: every evaluable tap of theirs is FORCEd
@@ -447,132 +359,57 @@ struct Screener {
         qn = 0;
         pend = 0u;
         lower32 = (float)a.ncc_threshold - 1e-6f;
-        n_forced = n_screened = n_prerej = n_prebad = 0;
-        use_box = false;
-        stage_phase = 0u;
-        box_addr = 0u;
-        box_x0 = box_y0 = 0;
-#if SR_SCREEN2_STAGE
-        box_addr = (unsigned)__cvta_generic_to_shared(&sm.box[0][0]);
-        if (lane == 0) mbar_init((unsigned)__cvta_generic_to_shared(&sm.mbar), 1u);
-#endif
+        n_forced = n_screened = 0;
         if (STATS && alive && all_slow && a.stats) atomicAdd(a.stats + 4, 1ull);
         __syncwarp();
     }
 
     // ---- FP32 screen -----------------------------------------------------------------------------------
-    // The (2R+1)^2 taps around element `idx` of the neighbour's FP32 plane (slots [FIRST, LAST)).
-    template <int FIRST = 0, int LAST = WN>
+    // The (2R+1)^2 taps around element `idx` of the neighbour's FP32 plane.
     __device__ __forceinline__ void load_window(const float *__restrict__ gplane, int idx, float (&g)[WN]) const {
         const int fp = PITCH ? PITCH : a.pitch_f;
-#if SR_SCREEN2_ABL == 3  // ablation: warp-aligned (broadcast) loads
-        const float *__restrict__ base = gplane + ((idx & ~31) + 2);
-#else
         const float *__restrict__ base = gplane + idx;
-#endif
-#if SR_SCREEN2_ABL == 1  // ablation: no window loads
 #pragma unroll
-        for (int i = FIRST; i < LAST; ++i) g[i] = __int_as_float(idx + i);
-#else
-#pragma unroll
-        for (int i = FIRST; i < LAST; ++i) {
+        for (int i = 0; i < WN; ++i) {
             const int k = screen2_slot_tap<R>(i);
             g[i] = base[(k / WS - R) * fp + (k % WS - R)];
         }
-#endif
     }
 
     // One window: ub = ncc32 + eps (SCREEN_FORCE when FP64 has to decide), lb = ncc32 - eps (SCREEN_SKIP
-    // then), eps (statistics).
+    // then), eps (statistics).  The taps go in pairs through one FFMA2 accumulator pair per sum; the three
+    // sums interleave, which keeps dependent FFMA2s three issue slots apart.
     __device__ __forceinline__ void eval_window(const float (&g)[WN], float &ub, float &lb, float &eps_out) const {
         constexpr int NP = WN / 2;  // WN is odd: NP pairs + one scalar tap
-        float c32, eps;
-        bool ok;
-        if (ONEPASS) {
-            // NACC accumulator pairs per sum; the three sums interleave, so even one pair per sum keeps
-            // dependent FFMA2s three issue slots apart
-            constexpr int NACC = SR_SCREEN2_NACC;
-            float2 S1p[NACC], Qp[NACC], Xp[NACC];
+        const float2 zero = make_float2(0.0f, 0.0f);
+        float2 S1p = zero, Qp = zero, Xp = zero;
 #pragma unroll
-            for (int i = 0; i < NACC; ++i) S1p[i] = Qp[i] = Xp[i] = make_float2(0.0f, 0.0f);
-            const float2 zero = make_float2(0.0f, 0.0f);
-#pragma unroll
-            for (int p = 0; p < NP; ++p) {
-                const float2 wv = make_float2(wtf[2 * p], wtf[2 * p + 1]), gv = make_float2(g[2 * p], g[2 * p + 1]);
-                S1p[p % NACC] = fma2(wv, gv, S1p[p % NACC]);
-#if SR_SCREEN2_ABL != 2  // ablation 2: loads + one accumulation only
-                const float2 pv = fma2(wv, gv, zero);
-                Qp[p % NACC] = fma2(pv, pv, Qp[p % NACC]);
-                Xp[p % NACC] = fma2(make_float2(c1f[2 * p], c1f[2 * p + 1]), gv, Xp[p % NACC]);
-#endif
-            }
-            float S1, Q, X;
-            if (NACC == 1) {
-                S1 = S1p[0].x + S1p[0].y;
-                Q = Qp[0].x + Qp[0].y;
-                X = Xp[0].x + Xp[0].y;
-            } else {
-                S1 = (S1p[0].x + S1p[1].x) + (S1p[0].y + S1p[1].y);
-                Q = (Qp[0].x + Qp[1].x) + (Qp[0].y + Qp[1].y);
-                X = (Xp[0].x + Xp[1].x) + (Xp[0].y + Xp[1].y);
-            }
-            {
-                const float pl = wtf[WN - 1] * g[WN - 1];
-                S1 += pl;
-                Q = fmaf(pl, pl, Q);
-                X = fmaf(c1f[WN - 1], g[WN - 1], X);
-            }
-            const float mR = S1 * inv_totWf;
-            const float s3 = fmaf(-k0, mR * mR, Q);
-            const float s1 = fmaf(-mR, k1, X);
-            float rs;
-            asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(s3));
-            c32 = s1 * rs;
-            eps = fmaf(Q * (rs * rs), e1, e0);  // e0 + e1 * kappa
-            // ill-conditioned or non-finite neighbour window, or a bar too wide to be first order: FP64 decides
-            ok = (s3 >= (float)WN) && (eps <= SCREEN_EPS_MAX);
-        } else {
-            float2 S1p[2] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
-#pragma unroll
-            for (int p = 0; p < NP; ++p)
-                S1p[p & 1] = fma2(make_float2(wtf[2 * p], wtf[2 * p + 1]), make_float2(g[2 * p], g[2 * p + 1]), S1p[p & 1]);
-            float S1 = (S1p[0].x + S1p[1].x) + (S1p[0].y + S1p[1].y);
-            S1 = fmaf(wtf[WN - 1], g[WN - 1], S1);
-            const float mR = S1 * inv_totWf;
-            const float2 nm = make_float2(-mR, -mR);
-            float2 s3p[2] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
-            float2 s1p[2] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
-#pragma unroll
-            for (int p = 0; p < NP; ++p) {
-                const float2 t = fma2(make_float2(wtf[2 * p], wtf[2 * p + 1]), make_float2(g[2 * p], g[2 * p + 1]), nm);
-                s3p[p & 1] = fma2(t, t, s3p[p & 1]);
-                s1p[p & 1] = fma2(make_float2(c1f[2 * p], c1f[2 * p + 1]), t, s1p[p & 1]);
-            }
-            float s3a = (s3p[0].x + s3p[1].x) + (s3p[0].y + s3p[1].y);
-            float s1 = (s1p[0].x + s1p[1].x) + (s1p[0].y + s1p[1].y);
-            {
-                const float t = fmaf(wtf[WN - 1], g[WN - 1], -mR);
-                s3a = fmaf(t, t, s3a);
-                s1 = fmaf(c1f[WN - 1], t, s1);
-            }
-            // inactive taps (w = dl = 0) contributed (-mR)^2 each to s3a and nothing to s1; the label is
-            // FORCEd when that correction exceeds SCREEN_CORR_MAX * s3 (relative error of s3 <= 15u * 101,
-            // inside SCREEN_EPS_LOOSE, which such pixels always use)
-            const float s3 = fmaf(-k0, mR * mR, s3a);
-            eps = (s3 >= 100.0f * WN) ? e0 : SCREEN_EPS_LOOSE;
-            float rs;
-            asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(s3));
-            c32 = s1 * rs;
-            ok = (s3 >= (float)WN) && (s3 < 1e30f) && (s3a <= (SCREEN_CORR_MAX + 1.0f) * s3);
+        for (int p = 0; p < NP; ++p) {
+            const float2 wv = make_float2(wtf[2 * p], wtf[2 * p + 1]), gv = make_float2(g[2 * p], g[2 * p + 1]);
+            S1p = fma2(wv, gv, S1p);
+            const float2 pv = fma2(wv, gv, zero);
+            Qp = fma2(pv, pv, Qp);
+            Xp = fma2(make_float2(c1f[2 * p], c1f[2 * p + 1]), gv, Xp);
         }
+        float S1 = S1p.x + S1p.y, Q = Qp.x + Qp.y, X = Xp.x + Xp.y;
+        {
+            const float pl = wtf[WN - 1] * g[WN - 1];
+            S1 += pl;
+            Q = fmaf(pl, pl, Q);
+            X = fmaf(c1f[WN - 1], g[WN - 1], X);
+        }
+        const float mR = S1 * inv_totWf;
+        const float s3 = fmaf(-k0, mR * mR, Q);
+        const float s1 = fmaf(-mR, k1, X);
+        float rs;
+        asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rs) : "f"(s3));
+        const float c32 = s1 * rs;
+        const float eps = fmaf(Q * (rs * rs), e1, e0);  // e0 + e1 * kappa
+        // ill-conditioned or non-finite neighbour window, or a bar too wide to be first order: FP64 decides
+        const bool ok = (s3 >= (float)WN) && (eps <= SCREEN_EPS_MAX);
         eps_out = eps;
-#if SR_SCREEN2_ABL  // ablations: the arithmetic stays alive, no label ever becomes a candidate
-        lb = SCREEN_SKIP;
-        ub = (ok && c32 > 1e30f) ? c32 + eps : SCREEN_SKIP;
-#else
         lb = ok ? c32 - eps : SCREEN_SKIP;
         ub = ok ? c32 + eps : SCREEN_FORCE;
-#endif
     }
 
     // Two windows at once, vectorised ACROSS the two labels: every FFMA2 carries tap i of both windows in its
@@ -589,11 +426,9 @@ struct Screener {
             const float2 gv = make_float2(gA[i], gB[i]);
             const float2 wv = make_float2(wtf[i], wtf[i]);
             S1 = fma2(gv, wv, S1);
-#if SR_SCREEN2_ABL != 2
             const float2 pv = fma2(gv, wv, zero);
             Q = fma2(pv, pv, Q);
             X = fma2(gv, make_float2(c1f[i], c1f[i]), X);
-#endif
         }
         const float2 mR = fma2(S1, make_float2(inv_totWf, inv_totWf), zero);
         const float2 mR2 = fma2(mR, mR, zero);
@@ -609,26 +444,20 @@ struct Screener {
         const bool okx = (s3.x >= (float)WN) && (eps.x <= SCREEN_EPS_MAX), oky = (s3.y >= (float)WN) && (eps.y <= SCREEN_EPS_MAX);
         eps_out[0] = eps.x;
         eps_out[1] = eps.y;
-#if SR_SCREEN2_ABL
-        lb[0] = lb[1] = SCREEN_SKIP;
-        ub[0] = (okx && c32.x > 1e30f) ? up.x : SCREEN_SKIP;
-        ub[1] = (oky && c32.y > 1e30f) ? up.y : SCREEN_SKIP;
-#else
         lb[0] = okx ? lo.x : SCREEN_SKIP;
         lb[1] = oky ? lo.y : SCREEN_SKIP;
         ub[0] = okx ? up.x : SCREEN_FORCE;
         ub[1] = oky ? up.y : SCREEN_FORCE;
-#endif
     }
 
-    // NL windows at once: independent chains of one basic block.
+    // NL = 1 or 2 windows at once (two: eval_window2).
     template <int NL>
     __device__ __forceinline__ void screen_n(const float *__restrict__ gplane, const int (&idx)[NL], float (&ub)[NL], float (&lb)[NL],
                                              float (&eps_out)[NL]) const {
         float g[NL][WN];
 #pragma unroll
         for (int n = 0; n < NL; ++n) load_window(gplane, idx[n], g[n]);
-        if (NL == 2 && ONEPASS && SR_SCREEN2_LV) {
+        if (NL == 2) {
             float ub2[2], lb2[2], ep2[2];
             eval_window2(g[0], g[NL - 1], ub2, lb2, ep2);
 #pragma unroll
@@ -670,196 +499,6 @@ struct Screener {
         }
     }
 
-    // Software-pipelined sweep of a chunk: while label l is evaluated from one register set, the window of
-    // label l + 1 is loaded into the other.  The loads of a label no longer sit in front of its own
-    // arithmetic (a load phase on the LSU followed by an FMA phase, which the warps of a scheduler run in
-    // step with each other), they ride along with the previous label's FFMA2s.
-    __device__ __forceinline__ void chunk_pipelined(const float *__restrict__ gplane, unsigned ra, unsigned ca, int nl) {
-        float gA[WN], gB[WN];
-        int idxA, idxB;
-        int32_t tapA = lds_b32(ra), tapB;
-        bool inA = decode_tap(tapA, idxA), inB;
-        load_window(gplane, idxA, gA);
-        unsigned bit = 1u;
-#pragma unroll 1
-        for (int l = 0; l < nl; l += 2, ra += 256u, ca += 256u, bit <<= 2) {
-            float ub, lb, eps;
-            tapB = (l + 1 < nl) ? lds_b32(ra + 128u) : TAP_NONE;
-            inB = decode_tap(tapB, idxB);
-            load_window(gplane, idxB, gB);
-            eval_window(gA, ub, lb, eps);
-            commit_label(inA, tapA, ub, lb, eps, ca, bit, l);
-            tapA = (l + 2 < nl) ? lds_b32(ra + 256u) : TAP_NONE;
-            inA = decode_tap(tapA, idxA);
-            load_window(gplane, idxA, gA);
-            eval_window(gB, ub, lb, eps);
-            commit_label(inB, tapB, ub, lb, eps, ca + 128u, bit << 1, l + 1);
-        }
-    }
-
-    // Two-level sweep of a chunk (5x5 windows).
-    //
-    // Level 1 looks at the SCREEN2_PRE_TAPS taps of subset A only and proves most labels hopeless.  With
-    // dl the (unit-norm) reference deviations and t = p - meanR the neighbour's, over the active taps:
-    //     ncc = (<dl_A, t_A> + <dl_B, t_B>) / sqrt(|t_A|^2 + |t_B|^2)      (B = the taps not looked at)
-    // Maximising over the unknown t_B and over the unknown mean meanR (t_A = p_A - meanR 1_A ranges over a
-    // line in the plane spanned by p_A and 1_A) leaves
-    //     ncc^2 <= 1 - dist^2(dl_A, span{p_A, 1_A}) = 1 - E_A (1 - rho_A^2),
-    // E_A = the energy of dl_A about its own mean (a per-pixel constant), rho_A = the plain correlation of
-    // dl_A and p_A.  A label cannot reach the current lower bound L of the winning cost, and is dropped, if
-    //     rho_A^2 < 1 - (1 - L^2) / E_A     <=>     num^2 < (E_A - (1 - L^2)) * den,
-    // num = sum_A dl p - (sum_A dl)(sum_A p) / n_A,  den = sum_A p^2 - (sum_A p)^2 / n_A.  The FP32 sums carry
-    // |dnum| <= 32u sqrt(q), |dden| <= 32u q (q = sum_A p^2; 10 terms, <= 6 roundings each plus the inputs'):
-    // the test is made with (1 + 1/64) num^2 + 65 (32u)^2 q >= (|num| + |dnum|)^2 on the left and
-    // den - 2e-6 q <= den - |dden| on the right.  SR_MATCH_STATS=1 evaluates every dropped label in full as
-    // well and counts the ones that would have been candidates (must be 0).
-    //
-    // Level 2: the labels that survive (a 16-bit mask per lane) are evaluated in full, each lane taking
-    // ITS next surviving label per round, so the number of full evaluations a warp runs per chunk is the
-    // largest survivor count of a lane, not the number of labels with a survivor somewhere in the warp.
-    __device__ __forceinline__ void chunk_prescreened(const float *__restrict__ gplane, const unsigned ra0, const unsigned ca0, int nl) {
-        constexpr int PRE = SCREEN2_PRE_TAPS;
-        const float KB = pre_E - (1.0f - lower32 * lower32) * 1.000001f;  // (lower32 only rises: a stale value is conservative)
-        unsigned pass = 0u, bit = 1u;
-        unsigned ra = ra0, ca = ca0;
-#pragma unroll 1
-        for (int l = 0; l < nl; ++l, ra += 128u, ca += 128u, bit <<= 1) {
-            const int32_t tap = lds_b32(ra);
-            int idx;
-            if (decode_tap(tap, idx)) {
-                float g[WN];
-                load_window<0, PRE>(gplane, idx, g);
-                float2 Ap = make_float2(0.0f, 0.0f), Qp = make_float2(0.0f, 0.0f), Xp = make_float2(0.0f, 0.0f);
-                const float2 zero = make_float2(0.0f, 0.0f);
-#pragma unroll
-                for (int p = 0; p < PRE / 2; ++p) {
-                    const float2 wv = make_float2(wtf[2 * p], wtf[2 * p + 1]), gv = make_float2(g[2 * p], g[2 * p + 1]);
-                    const float2 pv = fma2(wv, gv, zero);
-                    Ap = fma2(wv, gv, Ap);
-                    Qp = fma2(pv, pv, Qp);
-                    Xp = fma2(make_float2(c1f[2 * p], c1f[2 * p + 1]), gv, Xp);
-                }
-                const float av = Ap.x + Ap.y, q = Qp.x + Qp.y, x = Xp.x + Xp.y;
-                const float num = fmaf(-pre_sdl_n, av, x);
-                const float den = fmaf(-av * pre_inv_n, av, q);
-                const float lhs = fmaf(num * num, 1.0157f, 2.4e-10f * q);
-                const float rhs = KB * fmaf(-2e-6f, q, den);
-                const bool reject = (KB > 0.0f) && (lhs < rhs);
-                if (!reject) pass |= bit;
-                if (STATS && reject) {  // self-check: the full evaluation of a dropped label
-                    ++n_prerej;
-                    float ub, lb, eps;
-                    load_window<PRE, WN>(gplane, idx, g);
-                    eval_window(g, ub, lb, eps);
-                    if (ub >= lower32) ++n_prebad;
-                }
-            } else if (tap != TAP_NONE && alive) {  // window on the neighbour's border / FP64-only pixel
-                sts_f32(ca, SCREEN_FORCE);
-                pend |= bit;
-                if (STATS) ++n_forced;
-            }
-        }
-#pragma unroll 1
-        while (__any_sync(FULL, pass != 0u)) {
-            const bool has = pass != 0u;
-            const int l = has ? __ffs(pass) - 1 : 0;
-            pass &= pass - 1u;
-            const int32_t tap = lds_b32(ra0 + 128u * l);
-            int idx;
-            const bool interior = decode_tap(tap, idx) && has;
-            float g[WN], ub, lb, eps;
-            load_window(gplane, interior ? idx : R * (PITCH ? PITCH : a.pitch_f) + R, g);
-            eval_window(g, ub, lb, eps);
-            if (interior) commit_label(true, tap, ub, lb, eps, ca0 + 128u * l, 1u << l, l);
-        }
-    }
-
-#if SR_SCREEN2_STAGE
-    // north_star stage (1): "neighbour views staged in shared memory via TMA".  The warp's interior taps of a
-    // chunk span a band of the neighbour image; its bounding box (+ the window radius) is copied row by row
-    // with cp.async.bulk (the TMA engine; a row is one contiguous run, so no tensor map is needed), completion
-    // on an mbarrier, and the windows are read with LDS at immediate offsets.  A band that does not fit
-    // STAGE_BH x STAGE_BW falls back to the global loads for that chunk.
-    __device__ __forceinline__ void stage_chunk(const float *__restrict__ gplane, unsigned ra, int nl) {
-        const int fp = PITCH ? PITCH : a.pitch_f;
-        int xmin = 1 << 20, xmax = -1, ymin = 1 << 20, ymax = -1;
-#pragma unroll 4
-        for (int l = 0; l < nl; ++l) {
-            const int32_t tap = lds_b32(ra + 128u * l);
-            const int tx = tap & 0xffff, ty = (int)((uint32_t)tap >> 16);
-            if ((unsigned)(tx - R) < (unsigned)my_win_w && (unsigned)(ty - R) < (unsigned)a.win_h) {
-                xmin = min(xmin, tx);
-                xmax = max(xmax, tx);
-                ymin = min(ymin, ty);
-                ymax = max(ymax, ty);
-            }
-        }
-        xmin = __reduce_min_sync(FULL, xmin);
-        xmax = __reduce_max_sync(FULL, xmax);
-        ymin = __reduce_min_sync(FULL, ymin);
-        ymax = __reduce_max_sync(FULL, ymax);
-        use_box = false;
-        if (xmax < 0) return;
-        const int x0 = (xmin - R) & ~3, y0 = ymin - R;
-        const int bw = min(((xmax + R + 1 - x0) + 3) & ~3, fp - x0), bh = ymax + R + 1 - y0;
-        if (xmax + R + 1 - x0 > bw || bw > STAGE_BW || bh > STAGE_BH) return;
-        const unsigned mbar = (unsigned)__cvta_generic_to_shared(&sm.mbar);
-        // the box was last read through the generic proxy, the copies write it through the async proxy
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        if (lane == 0) mbar_expect_tx(mbar, (unsigned)(bh * bw * 4));
-        __syncwarp();
-        if (lane < bh) bulk_g2s(box_addr + (unsigned)(lane * STAGE_BW * 4), gplane + ((size_t)(y0 + lane) * fp + x0), (unsigned)(bw * 4), mbar);
-        while (!mbar_try_wait(mbar, stage_phase)) {
-        }
-        stage_phase ^= 1u;
-        use_box = true;
-        box_x0 = x0;
-        box_y0 = y0;
-    }
-    __device__ __forceinline__ void load_window_box(unsigned addr, float (&g)[WN]) const {
-#pragma unroll
-        for (int i = 0; i < WN; ++i) {
-            const int k = screen2_slot_tap<R>(i);
-            g[i] = lds_f32(addr + (unsigned)(((k / WS - R) * STAGE_BW + (k % WS - R)) * 4));
-        }
-    }
-    // labels<NL> with the windows read from the staged band
-    template <int NL>
-    __device__ __forceinline__ void labels_box(unsigned ra, unsigned ca, unsigned bit, int l) {
-        int32_t tap[NL];
-        unsigned addr[NL];
-        bool interior[NL], any = false;
-#pragma unroll
-        for (int n = 0; n < NL; ++n) {
-            tap[n] = lds_b32(ra + 128u * n);
-            const int tx = tap[n] & 0xffff, ty = (int)((uint32_t)tap[n] >> 16);
-            interior[n] = (unsigned)(tx - R) < (unsigned)my_win_w && (unsigned)(ty - R) < (unsigned)a.win_h;
-            const int off = interior[n] ? (ty - box_y0) * STAGE_BW + (tx - box_x0) : R * STAGE_BW + R;
-            addr[n] = box_addr + (unsigned)(off * 4);
-            any = any || interior[n];
-        }
-        float ub[NL], lb[NL], eps[NL];
-#pragma unroll
-        for (int n = 0; n < NL; ++n) ub[n] = lb[n] = eps[n] = 0.0f;
-        if (any) {
-            float g[NL][WN];
-#pragma unroll
-            for (int n = 0; n < NL; ++n) load_window_box(addr[n], g[n]);
-            if (NL == 2 && ONEPASS && SR_SCREEN2_LV) {
-                float ub2[2], lb2[2], ep2[2];
-                eval_window2(g[0], g[NL - 1], ub2, lb2, ep2);
-#pragma unroll
-                for (int n = 0; n < NL; ++n) ub[n] = ub2[n], lb[n] = lb2[n], eps[n] = ep2[n];
-            } else {
-#pragma unroll
-                for (int n = 0; n < NL; ++n) eval_window(g[n], ub[n], lb[n], eps[n]);
-            }
-        }
-#pragma unroll
-        for (int n = 0; n < NL; ++n) commit_label(interior[n], tap[n], ub[n], lb[n], eps[n], ca + 128u * n, bit << n, l + n);
-    }
-#endif
-
     // NL consecutive labels of a chunk: ring entries at shared addresses ra, ra + 128, ...; `bit` = mask bit
     // of the first.  A lane with at least one interior label evaluates all NL (the others at a safe address,
     // result discarded).
@@ -886,30 +525,13 @@ struct Screener {
     __device__ __forceinline__ void chunk(int j, int d0, int nl, int buf, const float *__restrict__ gplane) {
         unsigned ra = (unsigned)__cvta_generic_to_shared(&sm.tap_ring[buf][0][lane]);
         unsigned ca = (unsigned)__cvta_generic_to_shared(&sm.ub_ring[0][lane]);
-        if (SR_SCREEN2_PRE && ONEPASS && R == 2) {
-            chunk_prescreened(gplane, ra, ca, nl);
-        } else if (SR_SCREEN2_SWP && ONEPASS) {
-            chunk_pipelined(gplane, ra, ca, nl);
-        } else {
-            unsigned bit = 1u;
-            constexpr int NL = SR_SCREEN2_NL;
-            int l = 0;
-#if SR_SCREEN2_STAGE
-            stage_chunk(gplane, ra, nl);
-            if (use_box) {
+        unsigned bit = 1u;
+        int l = 0;
+        // two labels per iteration (independent chains, eval_window2), then an odd last label on its own
 #pragma unroll 1
-                for (; l + NL <= nl; l += NL, ra += 128u * NL, ca += 128u * NL, bit <<= NL) labels_box<NL>(ra, ca, bit, l);
+        for (; l + 2 <= nl; l += 2, ra += 256u, ca += 256u, bit <<= 2) labels<2>(gplane, ra, ca, bit, l);
 #pragma unroll 1
-                for (; l < nl; ++l, ra += 128u, ca += 128u, bit <<= 1) labels_box<1>(ra, ca, bit, l);
-            }
-#endif
-#pragma unroll 1
-            for (; l + NL <= nl; l += NL, ra += 128u * NL, ca += 128u * NL, bit <<= NL) labels<NL>(gplane, ra, ca, bit, l);
-            if (NL > 1) {
-#pragma unroll 1
-                for (; l < nl; ++l, ra += 128u, ca += 128u, bit <<= 1) labels<1>(gplane, ra, ca, bit, l);
-            }
-        }
+        for (; l < nl; ++l, ra += 128u, ca += 128u, bit <<= 1) labels<1>(gplane, ra, ca, bit, l);
         if (__any_sync(FULL, pend != 0u)) {
             const Screen2Cold r = screen2_process_pending<R, STATS>(a, sm, lane, first_pid, j, d0, buf, qn, pend, lower32);
             qn = r.qn;
@@ -925,7 +547,6 @@ struct Screener {
             atomicAdd(a.stats + 0, 1ull);
             atomicAdd(a.stats + 1, (unsigned long long)n_screened);
             atomicAdd(a.stats + 2, (unsigned long long)n_forced);
-            atomicAdd(a.stats + 7, (unsigned long long)n_prebad);  // labels the subset bound dropped although they were candidates
         }
         if (STATS && a.stats) {  // verifications are counted by the lane that ran them
             atomicAdd(a.stats + 3, (unsigned long long)sm.st_verified[lane]);
@@ -943,25 +564,15 @@ struct Screener {
     }
 };
 
-#ifndef SR_SCREEN2_TILE_ROWS
-#define SR_SCREEN2_TILE_ROWS 4  // warps per block: a block owns a 32 x TILE_ROWS tile of reference pixels (measured: 4 < 8 < 1)
-#endif
-#ifndef SR_SCREEN2_MINBLOCKS
-#define SR_SCREEN2_MINBLOCKS 4  // resident blocks per SM the register allocation must allow (x TILE_ROWS = 16 warps)
-#endif
-constexpr int SCREEN2_TILE_ROWS = SR_SCREEN2_TILE_ROWS;
+constexpr int SCREEN2_TILE_ROWS = 4;  // warps per block: a block owns a 32 x TILE_ROWS tile of reference pixels (measured: 4 < 8 < 1)
+constexpr int SCREEN2_MINBLOCKS = 4;  // resident blocks per SM the register allocation must allow (x TILE_ROWS = 16 warps)
 
 // Stand-alone form: the tap volume comes from HBM (label mode: build kernels; curve mode: the curve
 // rasteriser) through the two-stage cp.async ring.  The warps of a block are independent (nothing is
 // block-wide); they own the rows of a 32-pixel-wide tile so that their neighbour-image footprints overlap
 // in L1 (adjacent reference rows project to adjacent neighbour rows).  grid = (ceil(w/32), ceil(rows/TR)).
-#ifdef SR_SCREEN2_MAXNREG  // A/B: an explicit register cap instead of the one MINBLOCKS implies
-#define SR_SCREEN2_BOUNDS __maxnreg__(SR_SCREEN2_MAXNREG)
-#else
-#define SR_SCREEN2_BOUNDS __launch_bounds__(32 * SCREEN2_TILE_ROWS, SR_SCREEN2_MINBLOCKS)
-#endif
 template <int R, bool STATS, int PITCH>
-__global__ void SR_SCREEN2_BOUNDS match_mvs_screen2_kernel(const __grid_constant__ MatchArgs a) {
+__global__ void __launch_bounds__(32 * SCREEN2_TILE_ROWS, SCREEN2_MINBLOCKS) match_mvs_screen2_kernel(const __grid_constant__ MatchArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     Screen2Smem<STATS> &sm = reinterpret_cast<Screen2Smem<STATS> *>(smem_raw)[warp];

@@ -57,7 +57,7 @@ def test_cfg4_full_size_properties(cfg4, monkeypatch):
     ms, bs = stats
     assert bs["interpolated"] > 1e9 and bs["tap_mismatches"] == 0
     # every verified label inside its own error bar (one-pass screen: the bar follows the label's cancellation,
-    # e0 + e1 * kappa, typically 1e-5 .. 1e-4), and the subset bound (when compiled in) never dropped a candidate
+    # e0 + e1 * kappa, typically 1e-5 .. 1e-4), and the reserved slot 7 (prescreen_false_drops) reads 0
     assert ms["outside_error_bar"] == 0 and ms["max_screen_err"] < 1e-4 and ms["prescreen_false_drops"] == 0
     # screened path == all-FP64 kernel, same taps
     (i0, d0, b0), _ = _run(monkeypatch, cams, imgs, P, {"SR_MATCH_SCREEN": "0"})

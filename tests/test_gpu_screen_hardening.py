@@ -2,8 +2,8 @@
 own self-check counters read (SR_MATCH_STATS=1):
 
   * the FP32 screen's error bars (sr_screen2.cuh: eps = e0 + e1 * kappa per label) — every verified label
-    must lie inside its bar (`outside_error_bar == 0`), and the subset bound of the two-level sweep, when
-    compiled in, must never drop a candidate (`prescreen_false_drops == 0`);
+    must lie inside its bar (`outside_error_bar == 0`), and the reserved slot 7 of the counters reads 0
+    (`prescreen_false_drops == 0`, sr_b200.h);
   * the anchor interpolation of the refractive build (sr_build_refr.cuh) — with the switch on every
     interpolated label is also projected exactly, `tap_mismatches == 0`.
 
@@ -14,9 +14,8 @@ edges (support weights from 1 down to below the 1e-10 cut-off inside one window)
 compared with the oracle as everywhere else; the reference rule being protected is the candidate selection
 of stereo/multiviewstereo.cpp:589-602,654-660.
 
-Also here: the variants that must not change a single output bit — the two internal lanes
-(SR_LANES=1 vs the default), the one-launch pipeline (SR_PIPELINE=1) — and a context that is re-used with
-larger images while peak lists are kept."""
+Also here: the two internal lanes, which must not change a single output bit (SR_LANES=1 vs the default),
+and a context that is re-used with larger images while peak lists are kept."""
 import numpy as np
 import pytest
 
@@ -142,8 +141,7 @@ def test_bunny_inside_its_bars(monkeypatch):
 
 
 def _run_views(monkeypatch, env, cams, imgs, ms, P, order):
-    for k in ("SR_LANES", "SR_PIPELINE"):
-        monkeypatch.delenv(k, raising=False)
+    monkeypatch.delenv("SR_LANES", raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, str(v))
     c = capi.Context(0)
@@ -162,12 +160,12 @@ def _same(a, b):
         ((a[2] == b[2]) | (np.isnan(a[2]) & np.isnan(b[2]))).all()
 
 
-def test_lanes_and_pipeline_are_bit_invisible(monkeypatch):
+def test_lanes_are_bit_invisible(monkeypatch):
     cams, imgs, ms, _ = refractive_arc_scene(V=5, w=112, h=72, masks=True)
     P = T.default_params(True, 420.0, 580.0, 48)
     order = [0, 1, 2, 3, 4, 2, 2, 0]  # (the same view twice in a row lands on different lanes)
     base = _run_views(monkeypatch, {"SR_LANES": 1}, cams, imgs, ms, P, order)
-    for env in ({}, {"SR_LANES": 2}, {"SR_PIPELINE": 1}, {"SR_PIPELINE": 1, "SR_PIPE_LAG": 2, "SR_PIPE_RING_MB": 1}):
+    for env in ({}, {"SR_LANES": 2}):
         got = _run_views(monkeypatch, env, cams, imgs, ms, P, order)
         for v in range(len(cams)):
             assert _same(base[v], got[v]), (env, v)

@@ -69,7 +69,7 @@ def test_screen_kernel_shape(lib):
     ops = sass(lib, SCREEN)
     ffma2 = sum(1 for o in ops if "FFMA2" in o)
     assert ffma2 >= 50, f"label-vectorised window arithmetic missing ({ffma2} FFMA2)"
-    assert not [o for o in ops if "UBLKCP" in o], "TMA staging (SR_SCREEN2_STAGE) is an opt-in experiment, not the shipped build"
+    assert not [o for o in ops if "UBLKCP" in o], "bulk async copies (TMA) in the screen: window loads are plain LDG through L1"
     regs, stack, _ = resources(lib)[SCREEN]
     assert regs <= 128, "4 blocks of 128 threads per SM need <= 128 registers"
     assert stack <= 128, f"stack frame grew to {stack} B: spills in the label loop (112 B shipped)"
