@@ -35,7 +35,7 @@ struct BuildRefrArgs {
     int32_t *taps;               // [D][rows][w] for this neighbour
     int w, h, row0, rows, D, d_chunk;
     int mvs;
-    unsigned long long *check;   // optional [4] (SR_BUILD_CHECK=1): labels interpolated, guard fall-backs,
+    unsigned long long *check;   // optional [4] (SR_MATCH_STATS=1): labels interpolated, guard fall-backs,
                                  // interpolated labels whose tap differs from the exact projection (must be 0)
 };
 

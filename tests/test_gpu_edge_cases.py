@@ -130,18 +130,22 @@ def test_single_and_seven_neighbours(ctx):
 def test_bad_arguments_fail_loudly(ctx):
     cams, imgs, ms, _ = refractive_arc_scene(V=3, w=32, h=24, masks=False)
     ctx.set_views(cams, imgs, None)
-    ctx.set_params(T.default_params(True, 420.0, 580.0, 8))
-    with pytest.raises(capi.SrError):
-        ctx.run_view(0, [0])  # a view cannot be its own neighbour
-    with pytest.raises(capi.SrError):
-        ctx.run_view(5, [0])
     with pytest.raises(capi.SrError):
         ctx.set_params(T.default_params(True, 420.0, 580.0, 1))  # fewer than two labels
     with pytest.raises(capi.SrError):
         ctx.set_params(T.default_params(True, 420.0, 580.0, 8, radius=9))  # unsupported radius
-    with pytest.raises(capi.SrError):
+    for run in (ctx.run_view, ctx.run_view_curve):  # label and curve mode share their argument checks
+        ctx.set_params(T.default_params(True, 420.0, 580.0, 8))
+        with pytest.raises(capi.SrError):
+            run(0, [0])  # a view cannot be its own neighbour
+        with pytest.raises(capi.SrError):
+            run(5, [0])
+        ctx.set_params(T.default_params(True, 420.0, 580.0, 8, row_begin=10, row_end=10))
+        with pytest.raises(capi.SrError):
+            run(0, [1, 2])  # empty row range
         ctx.set_params(T.default_params(False, 420.0, 580.0, 8))
-        ctx.run_view(0, [1, 2])  # two-view selection takes exactly one neighbour
+        with pytest.raises(capi.SrError):
+            run(0, [1, 2])  # two-view selection takes exactly one neighbour
 
 
 def test_camera_only_views(ctx):

@@ -15,7 +15,8 @@ compared with the oracle as everywhere else; the reference rule being protected 
 of stereo/multiviewstereo.cpp:589-602,654-660.
 
 Also here: the two internal lanes, which must not change a single output bit (SR_LANES=1 vs the default),
-and a context that is re-used with larger images while peak lists are kept."""
+and a context that is re-used with larger and smaller images (peak lists kept, label mode on the lanes, curve
+mode)."""
 import numpy as np
 import pytest
 
@@ -140,17 +141,21 @@ def test_bunny_inside_its_bars(monkeypatch):
         c.close()
 
 
-def _run_views(monkeypatch, env, cams, imgs, ms, P, order):
-    monkeypatch.delenv("SR_LANES", raising=False)
-    for k, v in env.items():
-        monkeypatch.setenv(k, str(v))
-    c = capi.Context(0)
+def _views_out(c, cams, imgs, ms, P, order, mode="run_view"):
     c.set_views(cams, imgs, ms)
     c.set_params(P)
     nb = c.select_neighbours(3)
     for v in order:
-        c.run_view(v, nb[v])
-    out = [(c.depth_index(v).copy(), c.depth(v).copy(), c.best_cost(v).copy()) for v in range(len(cams))]
+        getattr(c, mode)(v, nb[v])
+    return [(c.depth_index(v).copy(), c.depth(v).copy(), c.best_cost(v).copy()) for v in range(len(cams))]
+
+
+def _run_views(monkeypatch, env, cams, imgs, ms, P, order, mode="run_view"):
+    monkeypatch.delenv("SR_LANES", raising=False)
+    for k, v in env.items():
+        monkeypatch.setenv(k, str(v))
+    c = capi.Context(0)
+    out = _views_out(c, cams, imgs, ms, P, order, mode)
     c.close()
     return out
 
@@ -171,8 +176,11 @@ def test_lanes_are_bit_invisible(monkeypatch):
             assert _same(base[v], got[v]), (env, v)
 
 
-def test_context_reused_with_larger_images_and_peaks():
-    """ADVICE r1: the peak-list buffer follows the image size (it used to keep its first allocation)."""
+def test_context_reused_with_larger_images_and_peaks(monkeypatch):
+    """The context's grow-only buffers follow the image size.  First the peak-list buffer (ADVICE r1: it used to
+    keep its first allocation) against the oracle; then label mode on the default lanes and curve mode, each
+    through small -> large -> small images and label counts in one context, bit for bit against a fresh
+    context of each size."""
     c = capi.Context(0)
     try:
         for (w, h) in [(48, 32), (96, 64)]:
@@ -191,3 +199,18 @@ def test_context_reused_with_larger_images_and_peaks():
             assert np.abs(out[..., 0][same] - pk[..., 0][same]).max() <= 1e-9
     finally:
         c.close()
+    monkeypatch.delenv("SR_LANES", raising=False)
+    for mode in ("run_view", "run_view_curve"):
+        c = capi.Context(0)
+        try:
+            for (w, h, D) in [(48, 32, 16), (96, 64, 24), (48, 32, 16)]:
+                cams, imgs, ms, _ = refractive_arc_scene(V=4, w=w, h=h, masks=True)
+                P = T.default_params(True, 420.0, 580.0, D)
+                order = [1, 2, 0, 1]  # (label mode: both lanes run views of every size)
+                got = _views_out(c, cams, imgs, ms, P, order, mode)
+                want = _run_views(monkeypatch, {}, cams, imgs, ms, P, order, mode)
+                assert (got[1][0] >= 0).mean() > 0.1
+                for v in range(len(cams)):
+                    assert _same(got[v], want[v]), (mode, w, h, v)
+        finally:
+            c.close()
