@@ -259,14 +259,14 @@ int launch_weights(sr_ctx *ctx, const ViewDev &v, int kind, int radius, double *
     const size_t npix = list_x ? (size_t)list_n : (size_t)rows * ctx->w;
     const unsigned gx = (unsigned)((npix + 127) / 128);
     const size_t smem = (size_t)(2 * radius + 1) * (2 * radius + 1) * 128 * sizeof(double);
+    // From r = 3 up the shared-memory grid ((2r+1)^2 * 128 doubles, 49 KB at r = 3) exceeds 48 KB: the grid
+    // is the thread's column of W.
     if (kind == SR_WEIGHT_ADAPTIVE)
         weights_adaptive_kernel<<<gx, 128, (radius + 1) * sizeof(double), st>>>(wa);
     else if (radius == 2)  // MultiViewStereo's window (multiviewstereo.cpp:91): sweeps unrolled
         weights_geodesic_kernel<true, 2><<<gx, 128, smem, st>>>(wa);
     else if (radius == 1)
         weights_geodesic_kernel<true, 1><<<gx, 128, smem, st>>>(wa);
-    else if (smem <= 48 * 1024)
-        weights_geodesic_kernel<true, 0><<<gx, 128, smem, st>>>(wa);
     else
         weights_geodesic_kernel<false, 0><<<gx, 128, 0, st>>>(wa);
     CKL();

@@ -619,11 +619,39 @@ __global__ void __launch_bounds__(128, (R <= 2) ? SR_MATCH_MINBLOCKS : 2) match_
     }
     const bool degenerate = (COST == SR_COST_SAD_TWOVIEW) ? (nact <= 4 || totW <= 1e-10) : (totW < 1e-10);
     const double dnact = (double)nact;
+    // Error bar of the one-pass NCC (fast_one) against the reference's two passes, in FP64 (u = 2^-53).
+    //   S1 = sum p, S2 = sum p^2, S3 = sum (w dl) g with p = w g over the lane's taps in two chains, then
+    //   S + T and the lane butterfly: at most M roundings per term.  With A = S2 + 2 |meanR S1| + nact meanR^2
+    //   (S1 = meanR totW, so A = S2 + (2 totW + nact) meanR^2) and kappa = A / s3:
+    //     |dS1| <= M u S1 (terms >= 0),  |dS2| <= M u S2,  |dS3| <= M u sum |dl p| <= M u sqrt(s2 S2)
+    //     meanR = S1 / totW: (M + 2) u relative;  s3 = S2 - 2 meanR S1 + nact meanR^2 (two roundings),
+    //     whose derivative in meanR is 2 (nact meanR - S1):      |ds3| <= (3M + 7) u A
+    //     SD = sum dl (one chain of <= 2M), |SD| <= sqrt(nact s2):  |d(meanR SD)| <= (3M + 3) u |meanR| sqrt(nact s2)
+    //     s1 = S3 - meanR SD:                                       |ds1| <= u sqrt(s2) [(M + 1) sqrt(S2) + (3M + 3) |meanR| sqrt(nact)]
+    //   rho = s1 / sqrt(s2 s3) with |rho| <= 1 (Cauchy-Schwarz), S2 <= A and nact meanR^2 <= A:
+    //     |drho| <= |ds1| / sqrt(s2 s3) + |ds3| / (2 s3) + |ds2| / (2 s2) + rsqrt and the last products
+    //            <= u [(4M + 4) sqrt(kappa) + (1.5M + 3.5) kappa + M + 4]
+    //            <= u [(3.5M + 5.5) kappa + 3M + 6]                     (sqrt(kappa) <= (1 + kappa) / 2)
+    //   and, as A = s3 + 4 totW meanR^2 = s3 + 4 meanR S1, the bar exceeds RHO_TOL iff
+    //     meanR S1 * 4 u (3.5M + 5.5) / (RHO_TOL - u (6.5M + 11.5)) > s3             (two instructions a label)
+    //   A label whose bar exceeds RHO_TOL (5e-11 on the 255-scaled two-view cost, half the reference's 1e-10
+    //   selection margin; the MVS NCC is then within 2e-13) returns NaN: slow_cost, the reference's two-pass
+    //   filter, decides.  The bar is a worst case, and the one-pass error is a few u kappa at most in practice
+    //   (measured on the CPU: <= 40 u kappa, r = 1..16), so RHO_TOL is set well above the observed errors to
+    //   keep the fallback rare: kappa stays near 1 under adaptive weights (the reference's w g - meanR keeps s3
+    //   large), under geodesic weights it is mostly below the ~20-30 the bar allows (flagged: < 1 % of the labels
+    //   of a textured rectified pair, 6 % at r = 2 on an arc scene), and flat or smooth neighbour windows under
+    //   geodesic weights (kappa in the hundreds to millions, where s3 is a true variance) are flagged whole.
+    constexpr int M = (TPL + 1) / 2 + 1 + ((G >= 2) + (G >= 4) + (G >= 8) + (G >= 16) + (G >= 32));
+    constexpr double U = 1.1102230246251565e-16, RHO_TOL = 5e-11 / 255.0;
+    constexpr double ERR_K = U * (3.5 * M + 5.5), ERR_ROOM = RHO_TOL - U * (6.5 * M + 11.5);
+    static_assert(ERR_ROOM > 0.0, "RHO_TOL below the rounding floor of the window");
+    constexpr double ERR_C = 4.0 * ERR_K / ERR_ROOM;  // flag iff ERR_C meanR S1 > s3
 
     // one label, fast path: whole neighbour window in bounds; one streaming pass over the taps.
-    // Returns NaN iff a neighbour tap was invalid (NaN) — then the exact tap filter (slow_cost)
-    // decides.  A legitimately evaluated cost is never NaN (two-view: NaN -> 120 as std::min
-    // does; MVS: q < 1e-10 -> 0).
+    // Returns NaN iff a neighbour tap was invalid (NaN), the NCC's error bar exceeds RHO_TOL or
+    // the two-view q is out of range — then the exact tap filter (slow_cost) decides.  A legitimately evaluated cost is never NaN
+    // (two-view: NaN -> 120 as std::min does; MVS: q < 1e-10 -> 0).
     auto fast_one = [&](const double *__restrict__ base) -> double {
         double S1 = 0.0, S2 = 0.0, S3 = 0.0, T1 = 0.0, T2 = 0.0, T3 = 0.0;
         if (G == 1) {
@@ -693,10 +721,14 @@ __global__ void __launch_bounds__(128, (R <= 2) ? SR_MATCH_MINBLOCKS : 2) match_
         const double s1 = fma(-meanR, SD, S3);
         const double s3 = fma(dnact * meanR, meanR, fma(-2.0 * meanR, S1, S2));
         const double q = s2 * s3;
-        if (COST == SR_COST_NCC_MVS) return (q < 1e-10) ? 0.0 : s1 * fast_rsqrt(q);
-        // two-view: 255*(1 - |s1|/sqrt(q)); q <= 0 or denormal takes the IEEE path (inf/NaN -> 120)
-        const double rs = (q > 1e-280 && q < 1e280) ? fast_rsqrt(q) : rsqrt(q);
-        const double v = 255.0 * (1.0 - fabs(s1) * rs);
+        if (COST == SR_COST_NCC_MVS) {
+            if (fma(ERR_C * meanR, S1, -s3) > 0.0) return qnan();  // error bar > RHO_TOL
+            return (q < 1e-10) ? 0.0 : s1 * fast_rsqrt(q);
+        }
+        // two-view: 255*(1 - |s1|/sqrt(q)); an error bar > RHO_TOL, or q <= 0, denormal or huge (the IEEE
+        // inf/NaN -> 120 cases): slow_cost
+        if (fma(ERR_C * meanR, S1, -s3) > 0.0 || !(q > 1e-280 && q < 1e280)) return qnan();
+        const double v = 255.0 * (1.0 - fabs(s1) * fast_rsqrt(q));
         return (v < 120.0) ? v : 120.0;
     };
 
