@@ -211,6 +211,19 @@ int sr_set_depth(sr_ctx *ctx, int view, const double *depth);
  * gray ramp, masked -> WHITE) or stereo/twoviewstereo.cpp:128-146 (HSV ramp).
  * RGBA8 w*h*4 out. */
 int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *rgba8_out);
+/* The coloured point cloud of `view`'s current depth map (the input of outputPLYFile,
+ * stereo/multiviewstereo.cpp:291-315).  For every pixel (x, y) whose depth d is finite and
+ * d + 1e-5 >= min_depth of the last sr_set_params: the intersection of
+ * Camera::unproject((x + .5) / image_scale, (y + .5) / image_scale) with the plane through C + d n,
+ * n = principleRay().direction() (pointFromDepth, :740-750; pixels whose intersection fails are
+ * skipped), and the pixel's R, G, B.  Points come in row-major pixel order, whatever wrote the map
+ * (a run, sr_cross_check, sr_set_depth, a gather) and whichever sentinels it holds.
+ * out_xyz = 3 * capacity doubles, out_rgb = 3 * capacity bytes, out_pixel = capacity pixel indices
+ * y * w + x (may be NULL).  *out_count receives the number of points; capacity 0 (pointers NULL)
+ * only counts.  SR_ERR_INVALID when capacity < count (*out_count is set, nothing else written);
+ * SR_ERR_STATE for a view without an image or before sr_set_params. */
+int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint8_t *out_rgb,
+                  int32_t *out_pixel, int64_t *out_count);
 
 /* ---- building blocks exposed for the C++ class API and the parity tests -----*/
 /* Camera::unproject on every pixel centre ((x+.5)/scale,(y+.5)/scale)

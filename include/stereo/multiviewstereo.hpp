@@ -8,6 +8,7 @@
 //   computeInitialEstimate (:524-662)     sr_run_view, MultiViewStereo selection over depth labels
 //   crossCheck (:666-729)                 sr_cross_check
 //   colourisation (:257-278, :381-395)    sr_get_depth_image
+//   point cloud (:291-315, :740-750)      sr_get_points (with setKeepPointCloud(true))
 // No CPU fallback: a missing CUDA device makes run() throw from sr_ctx_create.
 #ifndef SR_STEREO_MULTIVIEWSTEREO_HPP
 #define SR_STEREO_MULTIVIEWSTEREO_HPP
@@ -52,6 +53,8 @@ public:
         this->imageScale = imageScale;
         this->views.clear();
         peakPairs_.clear();
+        keptCloud_.clear();
+        cloudKept_ = false;
         inMemory_ = false;
         images.clear();
         masks.clear();
@@ -110,12 +113,18 @@ public:
     //! [h][w][9][2] (ncc, depth), ascending, padded with (0, -1); the last pair is the pixel's result
     //! before the cross-check.  Empty unless setKeepPeaks(true).
     const std::vector<double> &peakPairs(size_t viewIndex) const { return peakPairs_[viewIndex]; }
+    //! true: runTask() also computes every view's coloured point cloud on the GPU (sr_get_points) after the
+    //! cross-check, and pointCloud() returns it.  Off by default: the cloud costs a kernel, ~60 MB of copies
+    //! per 1080p view and the PLYPoint vector on every run.
+    void setKeepPointCloud(bool on) { keepPointCloud_ = on; }
     size_t numViews() const { return views.size(); }
     const std::vector<double> &depths(size_t viewIndex) const { return computedDepths[viewIndex]; }
     const std::vector<int32_t> &indices(size_t viewIndex) const { return depthIndices[viewIndex]; }
     const std::vector<std::vector<size_t> > &selectedNeighbours() const { return neighbours; }
-    //! Depth maps as a coloured point cloud (what the GUI's PLY export consumes).
+    //! Depth maps as a coloured point cloud (what the GUI's PLY export consumes), views in order, pixels
+    //! row-major.  The cloud the last run kept (setKeepPointCloud(true)), else unprojected here on the host.
     std::vector<PLYPoint> pointCloud() const {
+        if (cloudKept_) return keptCloud_;
         std::vector<PLYPoint> pts;
         for (size_t v = 0; v < views.size(); ++v) {
             const int w = images[v].width(), h = images[v].height();
@@ -134,6 +143,8 @@ public:
 
 protected:
     void runTask() {
+        keptCloud_.clear();
+        cloudKept_ = false;
         if ((!inMemory_ && (!project || !imageSet_)) || views.empty()) return;  // multiviewstereo.cpp:326-327
         const int V = (int)views.size();
         const int w = images[0].width(), h = images[0].height();
@@ -194,6 +205,7 @@ protected:
         stageUpdate("Constructing depth maps");
         fetch(s, w, h);
         coverage_after_ = coverage();
+        if (keepPointCloud_) keepPointCloud(s);
     }
 
 public:
@@ -229,6 +241,24 @@ private:
         }
     }
 
+    void keepPointCloud(sr_host::Session &s) {
+        std::vector<double> xyz;
+        std::vector<uint8_t> rgb;
+        for (size_t v = 0; v < views.size(); ++v) {
+            int64_t n = 0;
+            s.check(sr_get_points(s.get(), (int)v, 0, nullptr, nullptr, nullptr, &n), "sr_get_points");
+            if (n == 0) continue;
+            xyz.resize((size_t)n * 3);
+            rgb.resize((size_t)n * 3);
+            s.check(sr_get_points(s.get(), (int)v, n, xyz.data(), rgb.data(), nullptr, &n), "sr_get_points");
+            keptCloud_.reserve(keptCloud_.size() + (size_t)n);
+            for (size_t i = 0; i < (size_t)n; ++i)
+                keptCloud_.push_back(PLYPoint(Ray3d::Point(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]),
+                                              RGBA(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2])));
+        }
+        cloudKept_ = true;
+    }
+
     std::vector<double> coverage() const {
         std::vector<double> out;
         for (size_t v = 0; v < views.size(); ++v) {
@@ -254,6 +284,9 @@ private:
     std::vector<std::vector<int32_t> > depthIndices;
     std::vector<std::vector<double> > peakPairs_;
     std::vector<double> coverage_before_, coverage_after_;
+    std::vector<PLYPoint> keptCloud_;
+    bool keepPointCloud_ = false;
+    bool cloudKept_ = false;  // keptCloud_ belongs to the last run
     double minDepth, maxDepth;
     int numDepthLevels;
     double crossCheckThreshold;

@@ -25,7 +25,7 @@ EXPORTS = [
     "sr_set_stream", "sr_params_default", "sr_launch_count", "sr_set_profiling", "sr_get_stage_ms", "sr_get_match_stats", "sr_get_build_stats", "sr_set_views", "sr_set_params",
     "sr_run_view", "sr_run_view_curve", "sr_select_neighbours", "sr_cross_check", "sr_flush", "sr_synchronize",
     "sr_get_depth_index", "sr_get_depth", "sr_get_best_cost", "sr_get_cost_volume", "sr_get_peaks", "sr_set_depth",
-    "sr_get_depth_image", "sr_unproject_grid", "sr_project_points", "sr_compute_weights", "sr_calibration_residuals",
+    "sr_get_depth_image", "sr_get_points", "sr_unproject_grid", "sr_project_points", "sr_compute_weights", "sr_calibration_residuals",
     "sr_calibration_residuals_batch",
     "sr_comm_unique_id", "sr_comm_init", "sr_comm_allgather_views", "sr_comm_allgather_rows",
 ]
@@ -69,6 +69,8 @@ def lib():
         L.sr_ctx_destroy.argtypes = [C.c_void_p]
         L.sr_set_stream.argtypes = [C.c_void_p, C.c_void_p]
         L.sr_get_cost_volume.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        L.sr_get_points.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.POINTER(C.c_int64)]
         _LIB = L
     return _LIB
 
@@ -240,6 +242,18 @@ class Context:
         out = np.empty((self.h, self.w, 4), dtype=np.uint8)
         self._ck(self._L.sr_get_depth_image(self._h, view, int(mvs), _p(out)))
         return out
+
+    def points(self, view):
+        """The coloured point cloud of the view's depth map (sr_get_points): xyz (n, 3) float64, rgb (n, 3) uint8
+        and the pixel index y * w + x (n,) int32 of every point, in row-major pixel order."""
+        n = C.c_int64(0)
+        self._ck(self._L.sr_get_points(self._h, int(view), 0, None, None, None, C.byref(n)))
+        xyz = np.empty((n.value, 3), dtype=np.float64)
+        rgb = np.empty((n.value, 3), dtype=np.uint8)
+        pixel = np.empty(n.value, dtype=np.int32)
+        if n.value:
+            self._ck(self._L.sr_get_points(self._h, int(view), n.value, _p(xyz), _p(rgb), _p(pixel), C.byref(n)))
+        return xyz, rgb, pixel
 
     # -- building blocks -------------------------------------------------------------------
     def unproject_grid(self, view):

@@ -15,6 +15,7 @@
 #include "sr_match_dispatch.cuh"
 #include "sr_build_refr.cuh"
 #include "sr_curve.cuh"
+#include "sr_points.cuh"
 
 using namespace sr;
 
@@ -1062,11 +1063,66 @@ int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *out) {
     const size_t n = (size_t)ctx->w * ctx->h;
     rc = ensure_scratch(ctx, n * 4);
     if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    JOIN();  // the view may still be running on a lane
     depth_image_mvs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(
         ctx->views[view].depth, ctx->views[view].mask, (int)n, ctx->params.min_depth, ctx->params.max_depth,
         (uchar4 *)ctx->d_scratch);
     CKL();
     return d2h(ctx, out, ctx->d_scratch, n * 4);
+}
+
+int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint8_t *out_rgb, int32_t *out_pixel,
+                  int64_t *out_count) {
+    int rc = check_view(ctx, view);
+    if (rc) return rc;
+    if (!out_count || capacity < 0 || (capacity > 0 && (!out_xyz || !out_rgb)))
+        return fail(ctx, SR_ERR_INVALID, "sr_get_points: out_count, and out_xyz and out_rgb when capacity > 0, are required");
+    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    if (!ctx->views[view].have_image) return fail(ctx, SR_ERR_STATE, "the view was given no image in sr_set_views");
+    CK(cudaSetDevice(ctx->device));
+    JOIN();  // the view may still be running on a lane
+    const int h = ctx->h;
+    PointsArgs pa;
+    memset(&pa, 0, sizeof(pa));
+    pa.cam = ctx->cams[view];
+    pa.depth = ctx->views[view].depth;
+    pa.rgba = ctx->views[view].rgba;
+    pa.w = ctx->w;
+    pa.h = h;
+    pa.scale = ctx->params.image_scale;
+    pa.min_depth = ctx->params.min_depth;
+    // scratch: [row offsets][xyz][pixel][rgb]
+    const size_t off_bytes = ((size_t)(h + 1) * sizeof(long long) + 255) / 256 * 256;
+    auto count_points = [&]() -> int {
+        pa.offsets = (long long *)ctx->d_scratch;
+        points_count_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
+        CKL();
+        points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(pa.offsets, h);
+        CKL();
+        return SR_OK;
+    };
+    CKR(ensure_scratch(ctx, off_bytes));
+    CKR(count_points());
+    long long total = 0;
+    CKR(d2h(ctx, &total, pa.offsets + h, sizeof(total)));
+    *out_count = total;
+    if (capacity == 0 || total == 0) return SR_OK;
+    if (capacity < total) return fail(ctx, SR_ERR_INVALID, "sr_get_points: capacity is smaller than the number of points");
+    const size_t n = (size_t)total;
+    const size_t cap0 = ctx->scratch_cap;
+    CKR(ensure_scratch(ctx, off_bytes + n * (3 * sizeof(double) + sizeof(int32_t) + 3)));
+    if (ctx->scratch_cap != cap0) CKR(count_points());  // a new buffer: the offsets went with the old one
+    pa.xyz = (double *)((char *)ctx->d_scratch + off_bytes);
+    int32_t *d_pixel = (int32_t *)(pa.xyz + 3 * n);
+    pa.pixel = out_pixel ? d_pixel : nullptr;
+    pa.rgb = (uint8_t *)(d_pixel + n);
+    points_write_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
+    CKL();
+    CKR(d2h(ctx, out_xyz, pa.xyz, n * 3 * sizeof(double)));
+    CKR(d2h(ctx, out_rgb, pa.rgb, n * 3));
+    if (out_pixel) CKR(d2h(ctx, out_pixel, d_pixel, n * sizeof(int32_t)));
+    return SR_OK;
 }
 
 int sr_unproject_grid(sr_ctx *ctx, int view, double *out) {
