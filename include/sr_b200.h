@@ -186,7 +186,8 @@ int sr_flush(sr_ctx *ctx);
 int sr_synchronize(sr_ctx *ctx);
 
 /* ---- results (device -> host) ----------------------------------------------*/
-/* Depth-label index map, int32 w*h (extension, see SR_INDEX_*). */
+/* Depth-label index map, int32 w*h (extension, see SR_INDEX_*); after sr_mrf_select, the chosen
+ * peak-list slot 0..8. */
 int sr_get_depth_index(sr_ctx *ctx, int view, int32_t *out);
 /* computedDepth* / computedDepths[view] (stereo/twoviewstereo.hpp:41,
  * stereo/multiviewstereo.hpp:106-107): doubles with NaN / +INF / -1 sentinels. */
@@ -224,6 +225,47 @@ int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *rgba8_out);
  * SR_ERR_STATE for a view without an image or before sr_set_params. */
 int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint8_t *out_rgb,
                   int32_t *out_pixel, int64_t *out_count);
+
+/* ---- MRF stage on the peak lists --------------------------------------------*/
+/* The second stage of the multiple-hypothesis multi-view stereo the reference implements only in part
+ * (stereo/multiviewstereo.cpp:22-27): a Markov random field over the in-mask pixels (mask byte 255) of
+ * one view, 4-connected, whose labels are the 9 slots of a pixel's peak list plus U ("unknown").  A slot
+ * is a hypothesis when its ncc and depth are finite and it is not the padding (0, -1); other slots cannot
+ * be chosen.  With thr = ncc_threshold and step = (max_depth - min_depth) / (num_levels - 1) of the last
+ * sr_set_params:
+ *   D(k)    = max(0, (1 - ncc_k) / (1 - thr))            (FP64, rounded to FP32 once)
+ *   D(U)    = unknown_cost
+ *   V(k, l) = smooth_weight * min(|z_k - z_l|, smooth_trunc), z = depth / step (FP64, rounded to FP32
+ *             once and clamped to the finite FP32 range), so the truncation is in label steps
+ *   V(k, U) = V(U, k) = unknown_pair,  V(U, U) = 0.
+ * Solver: min-sum loopy belief propagation with FP32 messages on a checkerboard schedule; one iteration
+ * updates the messages sent by the pixels with (x + y) even, then by those with (x + y) odd.  The final
+ * label is argmin D + the four incoming messages; the highest hypothesis slot wins a tie, U loses every
+ * tie.  iterations = 0 gives the argmin of the unary term. */
+typedef struct sr_mrf_params {
+    int32_t iterations;    /* checkerboard iterations (both colours); 0 = argmin of the unary term */
+    double unknown_cost;   /* D(U)                                                    */
+    double smooth_weight;  /* V(k,l) = smooth_weight * min(|dz| / step, smooth_trunc) */
+    double smooth_trunc;   /* label steps                                             */
+    double unknown_pair;   /* V(k,U) = V(U,k); V(U,U) = 0                             */
+} sr_mrf_params;
+void sr_mrf_params_default(sr_mrf_params *p);
+/* Uploads peak lists for `view` (peaks = h*w*9*2 doubles, [pixel][k][ncc, depth], the layout of
+ * sr_get_peaks), replacing the lists the context keeps; sr_get_peaks and sr_mrf_select then read them.
+ * Any values are accepted: lists need not be sorted, and slots that are no hypothesis are skipped. */
+int sr_set_peaks(sr_ctx *ctx, int view, const double *peaks);
+/* Runs the MRF on the device-resident peak lists of `view` (a run with keep_cost_volume & 2, or
+ * sr_set_peaks) and writes that view's maps in place, on in-mask pixels only: depth = the chosen
+ * hypothesis's depth from the list (or -1 for U), best cost = its ncc (or 0), and the index map = the
+ * chosen SLOT 0..8 of the peak list (or SR_INDEX_NONE) -- after the MRF the index is a slot, not a depth
+ * label.  The peak lists are not modified.  out_energy (may be NULL) receives the energy of the final
+ * labelling: its FP32 unary and pairwise terms summed in FP64 in a fixed order.
+ * SR_ERR_STATE: no views, no params, or no peak lists for `view`.  SR_ERR_INVALID: a parameter negative
+ * or not finite, unknown_cost, unknown_pair or smooth_weight * smooth_trunc above 1e30 (which keeps every
+ * FP32 sum finite), iterations < 0, ncc_threshold >= 1 or not finite, max_depth <= min_depth, or a row
+ * band in the params (the MRF needs the whole view).  SR_ERR_CANCELLED: sr_request_cancel observed
+ * between iterations; the maps are then left as they were. */
+int sr_mrf_select(sr_ctx *ctx, int view, const sr_mrf_params *p, double *out_energy);
 
 /* ---- building blocks exposed for the C++ class API and the parity tests -----*/
 /* Camera::unproject on every pixel centre ((x+.5)/scale,(y+.5)/scale)

@@ -9,6 +9,7 @@
 //   crossCheck (:666-729)                 sr_cross_check
 //   colourisation (:257-278, :381-395)    sr_get_depth_image
 //   point cloud (:291-315, :740-750)      sr_get_points (with setKeepPointCloud(true))
+//   MRF stage on the peak lists (:22-27)  sr_mrf_select (with setMrf(true); the reference has no code for it)
 // No CPU fallback: a missing CUDA device makes run() throw from sr_ctx_create.
 #ifndef SR_STEREO_MULTIVIEWSTEREO_HPP
 #define SR_STEREO_MULTIVIEWSTEREO_HPP
@@ -40,6 +41,7 @@ class MultiViewStereo : public Task {
 public:
     MultiViewStereo() : minDepth(10), maxDepth(100), numDepthLevels(100), crossCheckThreshold(1), imageScale(1) {
         sr_params_default(&params_, 1);
+        sr_mrf_params_default(&mrfParams_);
     }
 
     void initialize(ProjectPtr project, ImageSetPtr imageSet, const std::vector<CameraPtr> &views, double minDepth,
@@ -117,6 +119,13 @@ public:
     //! cross-check, and pointCloud() returns it.  Off by default: the cloud costs a kernel, ~60 MB of copies
     //! per 1080p view and the PLYPoint vector on every run.
     void setKeepPointCloud(bool on) { keepPointCloud_ = on; }
+    //! true: after each view's search, choose every pixel's depth among its K = 9 peak-list hypotheses or
+    //! "unknown" with the MRF of sr_mrf_select (parameters: mrfParams()), before the cross-check.  The run
+    //! then keeps the peak lists (keep_cost_volume | 2), which takes it off the two lanes that overlap
+    //! consecutive views, and label mode evaluates every label with the all-FP64 match kernel.  indices()
+    //! then holds the chosen peak-list slot.  Off by default.
+    void setMrf(bool on) { mrf_ = on; }
+    sr_mrf_params &mrfParams() { return mrfParams_; }
     size_t numViews() const { return views.size(); }
     const std::vector<double> &depths(size_t viewIndex) const { return computedDepths[viewIndex]; }
     const std::vector<int32_t> &indices(size_t viewIndex) const { return depthIndices[viewIndex]; }
@@ -166,7 +175,9 @@ protected:
         params_.max_depth = maxDepth;
         params_.num_levels = numDepthLevels;
         params_.image_scale = imageScale;
-        s.check(sr_set_params(s.get(), &params_), "sr_set_params");
+        sr_params run = params_;
+        if (mrf_) run.keep_cost_volume |= 2;  // the MRF's input
+        s.check(sr_set_params(s.get(), &run), "sr_set_params");
 
         const int maxN = 3;  // NUM_NEIGHBOURING_VIEWS, multiviewstereo.cpp:96
         std::vector<int32_t> nb((size_t)V * maxN), cnt(V);
@@ -185,6 +196,7 @@ protected:
                     peakPairs_[v].resize((size_t)w * h * 18);
                     s.check(sr_get_peaks(s.get(), v, peakPairs_[v].data()), "sr_get_peaks");
                 }
+                if (mrf_) s.check(sr_mrf_select(s.get(), v, &mrfParams_, nullptr), "sr_mrf_select");
             } else {
                 // no neighbour was selected: the reference's loops find no candidate, which leaves -1 on the
                 // in-mask pixels and +INF on the others (multiviewstereo.cpp:559-565,604)
@@ -292,6 +304,8 @@ private:
     double crossCheckThreshold;
     double imageScale;
     sr_params params_;
+    sr_mrf_params mrfParams_;
+    bool mrf_ = false;
     int device_ = 0;
     bool inMemory_ = false;
     bool curveMode_ = true;   // the reference's live formulation; setCurveMode(false) = depth-label cost volume

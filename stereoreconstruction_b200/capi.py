@@ -9,7 +9,7 @@ import subprocess
 
 import numpy as np
 
-from .types import SrCamera, SrParams
+from .types import SrCamera, SrMrfParams, SrParams
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SR_LIB") or os.path.join(_PKG, "libsr_b200.so")  # SR_LIB: A/B kernel variants
@@ -24,9 +24,9 @@ EXPORTS = [
     "sr_ctx_create", "sr_ctx_destroy", "sr_last_error", "sr_request_cancel", "sr_clear_cancel",
     "sr_set_stream", "sr_params_default", "sr_launch_count", "sr_set_profiling", "sr_get_stage_ms", "sr_get_match_stats", "sr_get_build_stats", "sr_set_views", "sr_set_params",
     "sr_run_view", "sr_run_view_curve", "sr_select_neighbours", "sr_cross_check", "sr_flush", "sr_synchronize",
-    "sr_get_depth_index", "sr_get_depth", "sr_get_best_cost", "sr_get_cost_volume", "sr_get_peaks", "sr_set_depth",
+    "sr_get_depth_index", "sr_get_depth", "sr_get_best_cost", "sr_get_cost_volume", "sr_get_peaks", "sr_set_peaks", "sr_set_depth",
     "sr_get_depth_image", "sr_get_points", "sr_unproject_grid", "sr_project_points", "sr_compute_weights", "sr_calibration_residuals",
-    "sr_calibration_residuals_batch",
+    "sr_calibration_residuals_batch", "sr_mrf_params_default", "sr_mrf_select",
     "sr_comm_unique_id", "sr_comm_init", "sr_comm_allgather_views", "sr_comm_allgather_rows",
 ]
 
@@ -71,12 +71,26 @@ def lib():
         L.sr_get_cost_volume.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.sr_get_points.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.POINTER(C.c_int64)]
+        L.sr_mrf_params_default.argtypes = [C.POINTER(SrMrfParams)]
+        L.sr_mrf_params_default.restype = None
+        L.sr_mrf_select.argtypes = [C.c_void_p, C.c_int, C.POINTER(SrMrfParams), C.POINTER(C.c_double)]
         _LIB = L
     return _LIB
 
 
 class SrError(RuntimeError):
     pass
+
+
+def mrf_params_default(**kw):
+    """sr_mrf_params_default, with fields overridden by keyword."""
+    p = SrMrfParams()
+    lib().sr_mrf_params_default(C.byref(p))
+    for k, v in kw.items():
+        if not hasattr(p, k):
+            raise AttributeError(k)
+        setattr(p, k, v)
+    return p
 
 
 def _p(a):
@@ -133,6 +147,19 @@ class Context:
         out = np.empty((self.h, self.w, 9, 2), dtype=np.float64)
         self._ck(self._L.sr_get_peaks(self._h, int(view), _p(out)))
         return out
+
+    def set_peaks(self, view, peaks):
+        """Upload (h, w, 9, 2) float64 peak lists for the view (sr_set_peaks), the layout peaks() returns."""
+        pk = np.ascontiguousarray(peaks, dtype=np.float64)
+        assert pk.shape == (self.h, self.w, 9, 2), pk.shape
+        self._ck(self._L.sr_set_peaks(self._h, int(view), _p(pk)))
+
+    def mrf_select(self, view, params=None):
+        """sr_mrf_select on the view's peak lists (defaults when params is None); returns the labelling's energy."""
+        p = mrf_params_default() if params is None else params
+        e = C.c_double(0.0)
+        self._ck(self._L.sr_mrf_select(self._h, int(view), C.byref(p), C.byref(e)))
+        return e.value
 
     def build_stats(self):
         out = np.zeros(4, np.uint64)

@@ -16,6 +16,7 @@
 #include "sr_build_refr.cuh"
 #include "sr_curve.cuh"
 #include "sr_points.cuh"
+#include "sr_mrf.cuh"
 
 using namespace sr;
 
@@ -1123,6 +1124,104 @@ int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint
     CKR(d2h(ctx, out_rgb, pa.rgb, n * 3));
     if (out_pixel) CKR(d2h(ctx, out_pixel, d_pixel, n * sizeof(int32_t)));
     return SR_OK;
+}
+
+void sr_mrf_params_default(sr_mrf_params *p) {
+    if (!p) return;
+    p->iterations = MRF_DEFAULT_ITERATIONS;
+    p->unknown_cost = MRF_DEFAULT_UNKNOWN_COST;
+    p->smooth_weight = MRF_DEFAULT_SMOOTH_WEIGHT;
+    p->smooth_trunc = MRF_DEFAULT_SMOOTH_TRUNC;
+    p->unknown_pair = MRF_DEFAULT_UNKNOWN_PAIR;
+}
+
+int sr_set_peaks(sr_ctx *ctx, int view, const double *peaks) {
+    CKR(check_view(ctx, view));
+    if (!peaks) return fail(ctx, SR_ERR_INVALID, "sr_set_peaks: peaks is null");
+    const size_t n = (size_t)ctx->w * ctx->h;
+    std::vector<double> planar(n * 18);
+    for (size_t i = 0; i < n; ++i)  // [pixel][9][2] -> the device's [9][2][pixel]
+        for (int k = 0; k < 18; ++k) planar[(size_t)k * n + i] = peaks[i * 18 + k];
+    CK(cudaSetDevice(ctx->device));
+    JOIN();
+    ctx->peaks_view = -1;
+    CKR(grow(ctx, ctx->stream, ctx->d_peaks, ctx->peaks_cap, n * 18 * 8));
+    CK(cudaMemcpyAsync(ctx->d_peaks, planar.data(), n * 18 * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->peaks_view = view;
+    return SR_OK;
+}
+
+// A term of sr_mrf_params as the kernels use it: finite, >= 0, at most `cap`; +0 for a (signed) zero.
+static bool mrf_term(double v, double cap, float &out) {
+    if (!(v >= 0.0 && v <= cap)) return false;
+    out = v == 0.0 ? 0.0f : (float)v;
+    return true;
+}
+
+int sr_mrf_select(sr_ctx *ctx, int view, const sr_mrf_params *mp, double *out_energy) {
+    CKR(check_view(ctx, view));
+    if (!mp) return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: params is null");
+    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    if (ctx->peaks_view != view)
+        return fail(ctx, SR_ERR_STATE, "no peak lists for this view (run it with keep_cost_volume |= 2, or sr_set_peaks)");
+    const sr_params &P = ctx->params;
+    const int w = ctx->w, h = ctx->h;
+    const double step = (P.max_depth - P.min_depth) / (P.num_levels - 1.0);
+    if (P.num_levels < 2 || !(step > 0.0 && std::isfinite(step)))
+        return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: needs num_levels >= 2 and max_depth > min_depth");
+    if (!(P.ncc_threshold < 1.0 && std::isfinite(P.ncc_threshold)))
+        return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: ncc_threshold must be finite and < 1");
+    if (std::max(P.row_begin, 0) > 0 || (P.row_end > 0 && P.row_end < h))
+        return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: the MRF needs the whole view (a row band is set in the params)");
+    MrfArgs ma;
+    memset(&ma, 0, sizeof(ma));
+    const double cap = 1e30;
+    if (mp->iterations < 0 || !mrf_term(mp->unknown_cost, cap, ma.du) || !mrf_term(mp->smooth_weight, cap, ma.weight) ||
+        !mrf_term(mp->smooth_trunc, cap, ma.trunc) || !mrf_term(mp->unknown_pair, cap, ma.upair) ||
+        !(mp->smooth_weight * mp->smooth_trunc <= cap))
+            return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: iterations must be >= 0 and every term finite, >= 0 and at most "
+                                         "1e30 (smooth_weight * smooth_trunc too)");
+    CK(cudaSetDevice(ctx->device));
+    JOIN();
+    const size_t n = (size_t)w * h;
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    auto align = [](size_t b) { return (b + 255) / 256 * 256; };
+    // scratch: [messages 4*10*n][unary 9*n][z 9*n] floats, [labels n], [energy partials][energy]
+    const size_t msg_bytes = (size_t)4 * MRF_L * n * sizeof(float), slot_bytes = (size_t)MRF_K * n * sizeof(float);
+    const size_t lab_off = msg_bytes + 2 * slot_bytes, part_off = lab_off + align(n);
+    CKR(ensure_scratch(ctx, part_off + ((size_t)blocks + 1) * sizeof(double)));
+    char *base = (char *)ctx->d_scratch;
+    ViewDev &V = ctx->views[view];
+    ma.mask = V.mask;
+    ma.peaks = ctx->d_peaks;
+    ma.msg = (float *)base;
+    ma.unary = (float *)(base + msg_bytes);
+    ma.zs = (float *)(base + msg_bytes + slot_bytes);
+    ma.label = (uint8_t *)(base + lab_off);
+    ma.partial = (double *)(base + part_off);
+    ma.w = w;
+    ma.h = h;
+    mrf_prep_kernel<<<blocks, 256, 0, ctx->stream>>>(ma, 1.0 - P.ncc_threshold, step);
+    CKL();
+    CK(cudaMemsetAsync(ma.msg, 0, msg_bytes, ctx->stream));
+    const dim3 sweep_grid((unsigned)(((w + 1) / 2 + MRF_THREADS - 1) / MRF_THREADS), (unsigned)h);
+    for (int it = 0;; ++it) {
+        if (ctx->cancel.load()) return fail(ctx, SR_ERR_CANCELLED, "cancelled");
+        if (it == mp->iterations) break;
+        for (int colour = 0; colour < 2; ++colour) {
+            mrf_sweep_kernel<<<sweep_grid, MRF_THREADS, 0, ctx->stream>>>(ma, colour);
+            CKL();
+        }
+    }
+    mrf_label_kernel<<<blocks, 256, 0, ctx->stream>>>(ma, V.depth, V.best, V.index);
+    CKL();
+    if (!out_energy) return SR_OK;
+    mrf_energy_kernel<<<blocks, 256, 0, ctx->stream>>>(ma);
+    CKL();
+    mrf_sum_kernel<<<1, MRF_SUM_THREADS, 0, ctx->stream>>>(ma.partial, (int)blocks, ma.partial + blocks);
+    CKL();
+    return d2h(ctx, out_energy, ma.partial + blocks, sizeof(double));
 }
 
 int sr_unproject_grid(sr_ctx *ctx, int view, double *out) {

@@ -35,6 +35,13 @@ class SrParams(C.Structure):
     ]
 
 
+class SrMrfParams(C.Structure):
+    _fields_ = [
+        ("iterations", C.c_int32), ("unknown_cost", C.c_double), ("smooth_weight", C.c_double),
+        ("smooth_trunc", C.c_double), ("unknown_pair", C.c_double),
+    ]
+
+
 def default_params(multi_view, min_depth=10.0, max_depth=100.0, num_levels=100, **kw):
     """File-scope constants of the reference: two-view r=5 (stereo/twoviewstereo.cpp:64-80),
     MVS r=2 (stereo/multiviewstereo.cpp:90-102); both typedef GeodesicWeight."""
