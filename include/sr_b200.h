@@ -225,6 +225,32 @@ int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *rgba8_out);
  * SR_ERR_STATE for a view without an image or before sr_set_params. */
 int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint8_t *out_rgb,
                   int32_t *out_pixel, int64_t *out_count);
+/* One fused point cloud from the current depth maps of all V views, read as a snapshot (no map is
+ * modified, no view sees another's result; whatever wrote them does not matter), with the views'
+ * images and cameras and min_depth and image_scale s of the last sr_set_params.
+ *   1. Points.  The point of pixel (v, x, y) is the one sr_get_points gives it (finite d with
+ *      d + 1e-5 >= min_depth, the ray of Camera::unproject((x + .5) / s, (y + .5) / s) meeting the
+ *      plane through C + d n, n = prin_dir); a pixel whose intersection fails has none.
+ *   2. Agreement.  Let X be the point of source pixel p of view v.  Another view u agrees with p when
+ *      cam_project(u, X) succeeds, the projection times s is (x2, y2) with 0 <= x2 < w and
+ *      0 <= y2 < h, the pixel q = ((int)x2, (int)y2) of u has a point X_u (taken at q's centre), and
+ *      |X - X_u| is finite and < max_dist.  A(p) is the set of agreeing views, support(p) = |A(p)|.
+ *   3. Kept: support(p) >= min_views.
+ *   4. Emitted once: a kept p is emitted unless a view u in A(p) with u < v has its pixel q kept, so a
+ *      surface sample belongs to the lowest view that keeps it.  Agreement is not symmetric, so this is
+ *      not an exact one-to-one matching: two points of one surface sample can both be emitted.
+ *   5. Fused point: the FP64 sum of X and then the X_u of u in A(p) ascending, divided by
+ *      n = 1 + support(p); colour per channel (sum + n / 2) / n in integers over the same pixels.
+ *   6. Order: view-major, row-major pixel order within a view.
+ * With max_dist = 0 and min_views = 0 the result is the concatenation of sr_get_points over the views.
+ * The buffers follow sr_get_points: out_xyz = 3 * capacity doubles, out_rgb = 3 * capacity bytes,
+ * out_source = 2 * capacity int32 (view, y * w + x) (may be NULL); capacity 0 (pointers NULL) only
+ * counts.  SR_ERR_INVALID when capacity < count (*out_count is set, nothing else written), for a
+ * NULL out_count, a capacity > 0 without xyz or rgb, max_dist negative or not finite, or
+ * min_views < 0 (min_views > V - 1 is legal and gives no points).  SR_ERR_STATE without views or
+ * params, or when a view was given no image.  Scratch: 32 bytes per pixel of each view. */
+int sr_fuse_points(sr_ctx *ctx, double max_dist, int min_views, int64_t capacity, double *out_xyz,
+                   uint8_t *out_rgb, int32_t *out_source, int64_t *out_count);
 
 /* ---- MRF stage on the peak lists --------------------------------------------*/
 /* The second stage of the multiple-hypothesis multi-view stereo the reference implements only in part

@@ -10,6 +10,8 @@
 //   colourisation (:257-278, :381-395)    sr_get_depth_image
 //   point cloud (:291-315, :740-750)      sr_get_points (with setKeepPointCloud(true))
 //   MRF stage on the peak lists (:22-27)  sr_mrf_select (with setMrf(true); the reference has no code for it)
+//   fused point cloud of all views        sr_fuse_points (with setFusePointCloud(true); the reference only
+//                                         concatenates the views' clouds)
 // No CPU fallback: a missing CUDA device makes run() throw from sr_ctx_create.
 #ifndef SR_STEREO_MULTIVIEWSTEREO_HPP
 #define SR_STEREO_MULTIVIEWSTEREO_HPP
@@ -57,6 +59,7 @@ public:
         peakPairs_.clear();
         keptCloud_.clear();
         cloudKept_ = false;
+        fusedCloud_.clear();
         inMemory_ = false;
         images.clear();
         masks.clear();
@@ -125,6 +128,15 @@ public:
     //! consecutive views, and label mode evaluates every label with the all-FP64 match kernel.  indices()
     //! then holds the chosen peak-list slot.  Off by default.
     void setMrf(bool on) { mrf_ = on; }
+    //! true: runTask() also fuses the cross-checked depth maps of all views into one de-duplicated cloud on the
+    //! GPU (sr_fuse_points with max_dist = the cross-check threshold and min_views), and fusedPointCloud()
+    //! returns it: each surface sample once, averaged over the views that confirm it.  Off by default.
+    void setFusePointCloud(bool on, int minViews = 1) {
+        fusePointCloud_ = on;
+        fuseMinViews_ = minViews;
+    }
+    //! The fused cloud of the last run (setFusePointCloud(true)); empty otherwise.
+    const std::vector<PLYPoint> &fusedPointCloud() const { return fusedCloud_; }
     sr_mrf_params &mrfParams() { return mrfParams_; }
     size_t numViews() const { return views.size(); }
     const std::vector<double> &depths(size_t viewIndex) const { return computedDepths[viewIndex]; }
@@ -154,6 +166,7 @@ protected:
     void runTask() {
         keptCloud_.clear();
         cloudKept_ = false;
+        fusedCloud_.clear();
         if ((!inMemory_ && (!project || !imageSet_)) || views.empty()) return;  // multiviewstereo.cpp:326-327
         const int V = (int)views.size();
         const int w = images[0].width(), h = images[0].height();
@@ -218,6 +231,7 @@ protected:
         fetch(s, w, h);
         coverage_after_ = coverage();
         if (keepPointCloud_) keepPointCloud(s);
+        if (fusePointCloud_) fusePointCloud(s);
     }
 
 public:
@@ -271,6 +285,20 @@ private:
         cloudKept_ = true;
     }
 
+    void fusePointCloud(sr_host::Session &s) {
+        int64_t n = 0;
+        s.check(sr_fuse_points(s.get(), crossCheckThreshold, fuseMinViews_, 0, nullptr, nullptr, nullptr, &n), "sr_fuse_points");
+        if (n == 0) return;
+        std::vector<double> xyz((size_t)n * 3);
+        std::vector<uint8_t> rgb((size_t)n * 3);
+        s.check(sr_fuse_points(s.get(), crossCheckThreshold, fuseMinViews_, n, xyz.data(), rgb.data(), nullptr, &n),
+                "sr_fuse_points");
+        fusedCloud_.reserve((size_t)n);
+        for (size_t i = 0; i < (size_t)n; ++i)
+            fusedCloud_.push_back(PLYPoint(Ray3d::Point(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]),
+                                           RGBA(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2])));
+    }
+
     std::vector<double> coverage() const {
         std::vector<double> out;
         for (size_t v = 0; v < views.size(); ++v) {
@@ -299,6 +327,9 @@ private:
     std::vector<PLYPoint> keptCloud_;
     bool keepPointCloud_ = false;
     bool cloudKept_ = false;  // keptCloud_ belongs to the last run
+    std::vector<PLYPoint> fusedCloud_;
+    bool fusePointCloud_ = false;
+    int fuseMinViews_ = 1;
     double minDepth, maxDepth;
     int numDepthLevels;
     double crossCheckThreshold;

@@ -25,7 +25,7 @@ EXPORTS = [
     "sr_set_stream", "sr_params_default", "sr_launch_count", "sr_set_profiling", "sr_get_stage_ms", "sr_get_match_stats", "sr_get_build_stats", "sr_set_views", "sr_set_params",
     "sr_run_view", "sr_run_view_curve", "sr_select_neighbours", "sr_cross_check", "sr_flush", "sr_synchronize",
     "sr_get_depth_index", "sr_get_depth", "sr_get_best_cost", "sr_get_cost_volume", "sr_get_peaks", "sr_set_peaks", "sr_set_depth",
-    "sr_get_depth_image", "sr_get_points", "sr_unproject_grid", "sr_project_points", "sr_compute_weights", "sr_calibration_residuals",
+    "sr_get_depth_image", "sr_get_points", "sr_fuse_points", "sr_unproject_grid", "sr_project_points", "sr_compute_weights", "sr_calibration_residuals",
     "sr_calibration_residuals_batch", "sr_mrf_params_default", "sr_mrf_select",
     "sr_comm_unique_id", "sr_comm_init", "sr_comm_allgather_views", "sr_comm_allgather_rows",
 ]
@@ -71,6 +71,8 @@ def lib():
         L.sr_get_cost_volume.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.sr_get_points.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.POINTER(C.c_int64)]
+        L.sr_fuse_points.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.POINTER(C.c_int64)]
         L.sr_mrf_params_default.argtypes = [C.POINTER(SrMrfParams)]
         L.sr_mrf_params_default.restype = None
         L.sr_mrf_select.argtypes = [C.c_void_p, C.c_int, C.POINTER(SrMrfParams), C.POINTER(C.c_double)]
@@ -281,6 +283,19 @@ class Context:
         if n.value:
             self._ck(self._L.sr_get_points(self._h, int(view), n.value, _p(xyz), _p(rgb), _p(pixel), C.byref(n)))
         return xyz, rgb, pixel
+
+    def fuse_points(self, max_dist, min_views=1):
+        """One de-duplicated point cloud of all views' depth maps (sr_fuse_points): xyz (n, 3) float64, rgb (n, 3)
+        uint8 and the source (view, y * w + x) (n, 2) int32 of every point, view-major, row-major within a view."""
+        n = C.c_int64(0)
+        self._ck(self._L.sr_fuse_points(self._h, float(max_dist), int(min_views), 0, None, None, None, C.byref(n)))
+        xyz = np.empty((n.value, 3), dtype=np.float64)
+        rgb = np.empty((n.value, 3), dtype=np.uint8)
+        source = np.empty((n.value, 2), dtype=np.int32)
+        if n.value:
+            self._ck(self._L.sr_fuse_points(self._h, float(max_dist), int(min_views), n.value, _p(xyz), _p(rgb),
+                                            _p(source), C.byref(n)))
+        return xyz, rgb, source
 
     # -- building blocks -------------------------------------------------------------------
     def unproject_grid(self, view):

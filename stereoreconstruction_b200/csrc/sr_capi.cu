@@ -16,6 +16,7 @@
 #include "sr_build_refr.cuh"
 #include "sr_curve.cuh"
 #include "sr_points.cuh"
+#include "sr_fuse.cuh"
 #include "sr_mrf.cuh"
 
 using namespace sr;
@@ -113,6 +114,7 @@ struct sr_ctx {
     sr_camera *d_cams = nullptr;
     std::vector<ViewDev> views;
     double **d_depth_ptrs = nullptr;  // device array of per-view depth map pointers
+    uchar4 **d_rgba_ptrs = nullptr;   // device array of per-view image pointers
     sr_params params{};
     bool have_params = false;
     std::vector<double> depth_table;
@@ -222,6 +224,7 @@ void free_views(sr_ctx *c) {
     c->peaks_view = -1;  // peak lists belong to the image size they were computed at
     dfree(c->d_cams);
     dfree(c->d_depth_ptrs);
+    dfree(c->d_rgba_ptrs);
     free_scratch(c->s);  // sized for the old images
 }
 
@@ -544,10 +547,16 @@ int sr_set_views(sr_ctx *ctx, int V, const sr_camera *cams, const uint8_t *const
             }
             CK(cudaMalloc(&ctx->d_cams, sizeof(sr_camera) * V));
             CK(cudaMalloc(&ctx->d_depth_ptrs, sizeof(double *) * V));
+            CK(cudaMalloc(&ctx->d_rgba_ptrs, sizeof(uchar4 *) * V));
             CKR(grow(ctx, ctx->stream, ctx->s.rays, ctx->s.rays_cap, n * 6 * 8));
             std::vector<double *> ptrs(V);
-            for (int i = 0; i < V; ++i) ptrs[i] = ctx->views[i].depth;
+            std::vector<uchar4 *> rgba_ptrs(V);
+            for (int i = 0; i < V; ++i) {
+                ptrs[i] = ctx->views[i].depth;
+                rgba_ptrs[i] = ctx->views[i].rgba;
+            }
             CK(cudaMemcpyAsync(ctx->d_depth_ptrs, ptrs.data(), sizeof(double *) * V, cudaMemcpyHostToDevice, ctx->stream));
+            CK(cudaMemcpyAsync(ctx->d_rgba_ptrs, rgba_ptrs.data(), sizeof(uchar4 *) * V, cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaStreamSynchronize(ctx->stream));
             return SR_OK;
         }();
@@ -1123,6 +1132,74 @@ int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint
     CKR(d2h(ctx, out_xyz, pa.xyz, n * 3 * sizeof(double)));
     CKR(d2h(ctx, out_rgb, pa.rgb, n * 3));
     if (out_pixel) CKR(d2h(ctx, out_pixel, d_pixel, n * sizeof(int32_t)));
+    return SR_OK;
+}
+
+int sr_fuse_points(sr_ctx *ctx, double max_dist, int min_views, int64_t capacity, double *out_xyz, uint8_t *out_rgb,
+                   int32_t *out_source, int64_t *out_count) {
+    if (!ctx) return SR_ERR_INVALID;
+    if (!out_count || capacity < 0 || (capacity > 0 && (!out_xyz || !out_rgb)))
+        return fail(ctx, SR_ERR_INVALID, "sr_fuse_points: out_count, and out_xyz and out_rgb when capacity > 0, are required");
+    if (!(max_dist >= 0.0 && std::isfinite(max_dist)) || min_views < 0)
+        return fail(ctx, SR_ERR_INVALID, "sr_fuse_points: max_dist must be finite and >= 0, min_views >= 0");
+    if (ctx->V == 0) return fail(ctx, SR_ERR_STATE, "sr_set_views has not been called");
+    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    for (const ViewDev &v : ctx->views)
+        if (!v.have_image) return fail(ctx, SR_ERR_STATE, "sr_fuse_points: a view was given no image in sr_set_views");
+    CK(cudaSetDevice(ctx->device));
+    JOIN();  // a view may still be running on a lane
+    const int rows = ctx->V * ctx->h;
+    const size_t N = (size_t)ctx->V * ctx->w * ctx->h;
+    auto align = [](size_t b) { return (b + 255) / 256 * 256; };
+    FuseArgs fa;
+    memset(&fa, 0, sizeof(fa));
+    fa.cams = ctx->d_cams;
+    fa.depth = ctx->d_depth_ptrs;
+    fa.rgba = ctx->d_rgba_ptrs;
+    fa.V = ctx->V;
+    fa.w = ctx->w;
+    fa.h = ctx->h;
+    fa.scale = ctx->params.image_scale;
+    fa.min_depth = ctx->params.min_depth;
+    fa.max_dist = max_dist;
+    fa.min_views = min_views;
+    // scratch: [row offsets][fused xyz planes][support][rgbe], then the points' [xyz][source][rgb]
+    const size_t off_bytes = align((size_t)(rows + 1) * sizeof(long long));
+    const size_t pix_bytes = off_bytes + N * (3 * sizeof(double) + sizeof(int32_t) + sizeof(uint32_t));
+    auto count_points = [&]() -> int {
+        char *base = (char *)ctx->d_scratch;
+        fa.offsets = (long long *)base;
+        fa.fxyz = (double *)(base + off_bytes);
+        fa.support = (int32_t *)(fa.fxyz + 3 * N);
+        fa.rgbe = (uint32_t *)(fa.support + N);
+        fuse_support_kernel<<<(unsigned)((N + FUSE_THREADS - 1) / FUSE_THREADS), FUSE_THREADS, 0, ctx->stream>>>(fa);
+        CKL();
+        fuse_emit_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
+        CKL();
+        points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(fa.offsets, rows);
+        CKL();
+        return SR_OK;
+    };
+    CKR(ensure_scratch(ctx, pix_bytes));
+    CKR(count_points());
+    long long total = 0;
+    CKR(d2h(ctx, &total, fa.offsets + rows, sizeof(total)));
+    *out_count = total;
+    if (capacity == 0 || total == 0) return SR_OK;
+    if (capacity < total) return fail(ctx, SR_ERR_INVALID, "sr_fuse_points: capacity is smaller than the number of points");
+    const size_t n = (size_t)total;
+    const size_t cap0 = ctx->scratch_cap;
+    CKR(ensure_scratch(ctx, pix_bytes + n * (3 * sizeof(double) + 2 * sizeof(int32_t) + 3)));
+    if (ctx->scratch_cap != cap0) CKR(count_points());  // a new buffer: the scratch went with the old one
+    fa.xyz = (double *)((char *)ctx->d_scratch + pix_bytes);
+    int32_t *d_source = (int32_t *)(fa.xyz + 3 * n);
+    fa.source = out_source ? d_source : nullptr;
+    fa.rgb = (uint8_t *)(d_source + 2 * n);
+    fuse_write_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
+    CKL();
+    CKR(d2h(ctx, out_xyz, fa.xyz, n * 3 * sizeof(double)));
+    CKR(d2h(ctx, out_rgb, fa.rgb, n * 3));
+    if (out_source) CKR(d2h(ctx, out_source, d_source, n * 2 * sizeof(int32_t)));
     return SR_OK;
 }
 

@@ -16,7 +16,7 @@
 namespace sr {
 
 constexpr int POINTS_THREADS = 256;
-constexpr int POINTS_SCAN_THREADS = 1024;  // sr_set_views allows 16384 rows: at most 16 per scan thread
+constexpr int POINTS_SCAN_THREADS = 1024;  // any number of rows: fusion (sr_fuse.cuh) scans the rows of all V views
 
 struct PointsArgs {
     sr_camera cam;
@@ -30,13 +30,18 @@ struct PointsArgs {
     int32_t *pixel;       // [points] y * w + x, or null
 };
 
-// The pixel's point, if it has one: the filter and plane of MultiViewStereo::pointCloud.
-__device__ __forceinline__ bool point_of_pixel(const PointsArgs &a, int x, int y, d3 &p) {
-    const double d = a.depth[(size_t)y * a.w + x];
-    if (!isfinite(d) || d + 1e-5 < a.min_depth) return false;
+// The point of pixel (x, y) of a view with camera `cam` and depth map `depth` (row pitch w), if it has one: the
+// filter and plane of MultiViewStereo::pointCloud.
+__device__ __forceinline__ bool point_of_pixel(const sr_camera &cam, const double *depth, int w, int x, int y, double scale,
+                                               double min_depth, d3 &p) {
+    const double d = depth[(size_t)y * w + x];
+    if (!isfinite(d) || d + 1e-5 < min_depth) return false;
     d3 src, dir;
-    cam_unproject(a.cam, (x + 0.5) / a.scale, (y + 0.5) / a.scale, src, dir);
-    return point_from_depth(src, dir, ld3(a.cam.prin_dir), ld3(a.cam.C), d, p);
+    cam_unproject(cam, (x + 0.5) / scale, (y + 0.5) / scale, src, dir);
+    return point_from_depth(src, dir, ld3(cam.prin_dir), ld3(cam.C), d, p);
+}
+__device__ __forceinline__ bool point_of_pixel(const PointsArgs &a, int x, int y, d3 &p) {
+    return point_of_pixel(a.cam, a.depth, a.w, x, y, a.scale, a.min_depth, p);
 }
 
 __global__ void __launch_bounds__(POINTS_THREADS) points_count_kernel(const PointsArgs a) {
@@ -59,8 +64,8 @@ __device__ __forceinline__ long long warp_inclusive_sum(long long v, int lane) {
     return v;
 }
 
-// In place: offsets[r] = sum of the counts of rows < r, offsets[h] = sum of all.  Each thread owns a run of
-// consecutive rows.
+// In place: offsets[r] = sum of the counts of rows < r, offsets[h] = sum of all (h: any number of rows).  Each
+// thread owns a run of consecutive rows.
 __global__ void __launch_bounds__(POINTS_SCAN_THREADS) points_scan_kernel(long long *offsets, int h) {
     __shared__ long long warp_base[POINTS_SCAN_THREADS / 32];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -85,25 +90,34 @@ __global__ void __launch_bounds__(POINTS_SCAN_THREADS) points_scan_kernel(long l
     if (threadIdx.x == POINTS_SCAN_THREADS - 1) offsets[h] = run;
 }
 
+// Compaction of one POINTS_THREADS-wide chunk of a row: the number of keeping threads of the block before this
+// one, in thread order; `chunk` receives the block's total.  The caller synchronises before reusing warp_count.
+__device__ __forceinline__ int chunk_rank(bool keep, int *warp_count, int &chunk) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const unsigned ballot = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) warp_count[wid] = __popc(ballot);
+    __syncthreads();
+    int before = __popc(ballot & ((1u << lane) - 1u));
+    chunk = 0;
+#pragma unroll
+    for (int k = 0; k < POINTS_THREADS / 32; ++k) {
+        const int c = warp_count[k];
+        if (k < wid) before += c;
+        chunk += c;
+    }
+    return before;
+}
+
 __global__ void __launch_bounds__(POINTS_THREADS) points_write_kernel(const PointsArgs a) {
     __shared__ int warp_count[POINTS_THREADS / 32];
     const int y = blockIdx.x;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     long long base = a.offsets[y];
     for (int x0 = 0; x0 < a.w; x0 += POINTS_THREADS) {
         const int x = x0 + threadIdx.x;
         d3 p;
         const bool keep = x < a.w && point_of_pixel(a, x, y, p);
-        const unsigned ballot = __ballot_sync(0xffffffffu, keep);
-        if (lane == 0) warp_count[wid] = __popc(ballot);
-        __syncthreads();
-        int before = __popc(ballot & ((1u << lane) - 1u)), chunk = 0;
-#pragma unroll
-        for (int k = 0; k < POINTS_THREADS / 32; ++k) {
-            const int c = warp_count[k];
-            if (k < wid) before += c;
-            chunk += c;
-        }
+        int chunk;
+        const int before = chunk_rank(keep, warp_count, chunk);
         if (keep) {
             const long long o = base + before;
             const size_t i = (size_t)y * a.w + x;
