@@ -198,8 +198,6 @@ int sr_get_best_cost(sr_ctx *ctx, int view, double *out);
  * [nbr][d][row - row_begin][x] (label-major planes, the layout the kernels stream);
  * NaN where the label could not be evaluated. */
 int sr_get_cost_volume(sr_ctx *ctx, float *out, size_t out_elems);
-/* Replaces depth upload for cross-check under view sharding (each rank receives
- * the other ranks' depth maps before sr_cross_check). */
 /* The K = 9 largest (ncc, depth) pairs of every pixel of the last sr_run_view or
  * sr_run_view_curve with keep_cost_volume & 2, ascending, padded with (0, -1):
  * CostFunction::peakPairs, the input of the reference's MRF stage
@@ -207,10 +205,13 @@ int sr_get_cost_volume(sr_ctx *ctx, float *out, size_t out_elems);
  * [pixel][k][ncc, depth]; in curve mode depth is the z of the rays' closest approach (:583-588).
  * Evaluates every candidate in FP64. */
 int sr_get_peaks(sr_ctx *ctx, int view, double *out);
+/* Replaces depth upload for cross-check under view sharding (each rank receives
+ * the other ranks' depth maps before sr_cross_check). */
 int sr_set_depth(sr_ctx *ctx, int view, const double *depth);
-/* colorFromDepth + depthMap(view): stereo/multiviewstereo.cpp:257-286 (mvs != 0,
- * gray ramp, masked -> WHITE) or stereo/twoviewstereo.cpp:128-146 (HSV ramp).
- * RGBA8 w*h*4 out. */
+/* colorFromDepth + depthMap(view) of stereo/multiviewstereo.cpp:257-286: gray ramp,
+ * masked -> WHITE.  RGBA8 w*h*4 out.  mvs must be nonzero: mvs == 0 returns SR_ERR_INVALID,
+ * because the two-view HSV ramp (stereo/twoviewstereo.cpp:128-146, QColor semantics) is
+ * coloured on the host by the two-view class. */
 int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *rgba8_out);
 /* The coloured point cloud of `view`'s current depth map (the input of outputPLYFile,
  * stereo/multiviewstereo.cpp:291-315).  For every pixel (x, y) whose depth d is finite and
@@ -301,9 +302,6 @@ int sr_unproject_grid(sr_ctx *ctx, int view, double *out_rays);
  * doubles, out_ok = n flags. */
 int sr_project_points(sr_ctx *ctx, int view, int n, const double *xyz, double *out_xy,
                       int32_t *out_ok);
-/* AdaptiveWeight/GeodesicWeight::init_weights for n window centres
- * (stereo/adaptiveweight.cpp:47-58, stereo/geodesicweight.cpp:59-131):
- * out = n * (2r+1)^2 doubles, [row+r][col+r] as operator()(row,col) indexes. */
 /* The residual of the refractive-interface calibration, RefractiveCalibrationFunction::diff
  * (stereo/refractioncalibration.cpp:175-201), for n correspondences: view_pairs = 2n camera
  * indices into cams[num_cams], pixels = n * (x1, y1, x2, y2); out[i] = distance of the two
@@ -319,6 +317,9 @@ int sr_calibration_residuals(sr_ctx *ctx, int num_cams, const sr_camera *cams, i
  * is the caller. */
 int sr_calibration_residuals_batch(sr_ctx *ctx, int num_models, int num_cams, const sr_camera *cams,
                                    int n, const int32_t *view_pairs, const double *pixels, double *out);
+/* AdaptiveWeight/GeodesicWeight::init_weights for n window centres
+ * (stereo/adaptiveweight.cpp:47-58, stereo/geodesicweight.cpp:59-131):
+ * out = n * (2r+1)^2 doubles, [row+r][col+r] as operator()(row,col) indexes. */
 int sr_compute_weights(sr_ctx *ctx, int view, int weight_kind, int radius, int n,
                        const int32_t *cx, const int32_t *cy, double *out);
 

@@ -277,10 +277,7 @@ private:
             xyz.resize((size_t)n * 3);
             rgb.resize((size_t)n * 3);
             s.check(sr_get_points(s.get(), (int)v, n, xyz.data(), rgb.data(), nullptr, &n), "sr_get_points");
-            keptCloud_.reserve(keptCloud_.size() + (size_t)n);
-            for (size_t i = 0; i < (size_t)n; ++i)
-                keptCloud_.push_back(PLYPoint(Ray3d::Point(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]),
-                                              RGBA(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2])));
+            appendPoints(keptCloud_, xyz, rgb, (size_t)n);
         }
         cloudKept_ = true;
     }
@@ -293,10 +290,16 @@ private:
         std::vector<uint8_t> rgb((size_t)n * 3);
         s.check(sr_fuse_points(s.get(), crossCheckThreshold, fuseMinViews_, n, xyz.data(), rgb.data(), nullptr, &n),
                 "sr_fuse_points");
-        fusedCloud_.reserve((size_t)n);
-        for (size_t i = 0; i < (size_t)n; ++i)
-            fusedCloud_.push_back(PLYPoint(Ray3d::Point(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]),
-                                           RGBA(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2])));
+        appendPoints(fusedCloud_, xyz, rgb, (size_t)n);
+    }
+
+    // The first n points of the xyz / rgb arrays (3 values a point) of sr_get_points or sr_fuse_points, as PLYPoints.
+    static void appendPoints(std::vector<PLYPoint> &cloud, const std::vector<double> &xyz, const std::vector<uint8_t> &rgb,
+                             size_t n) {
+        cloud.reserve(cloud.size() + n);
+        for (size_t i = 0; i < n; ++i)
+            cloud.push_back(PLYPoint(Ray3d::Point(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]),
+                                     RGBA(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2])));
     }
 
     std::vector<double> coverage() const {

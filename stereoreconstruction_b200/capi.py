@@ -272,30 +272,29 @@ class Context:
         self._ck(self._L.sr_get_depth_image(self._h, view, int(mvs), _p(out)))
         return out
 
+    def _count_then_fill(self, call, extra_shape):
+        """Both calls of a count-then-fill entry point: call(capacity, xyz, rgb, extra, out_count) once with capacity
+        0 to count, then into arrays of that size.  Returns xyz (n, 3) float64, rgb (n, 3) uint8 and the int32
+        per-point array of shape (n, *extra_shape)."""
+        n = C.c_int64(0)
+        self._ck(call(0, None, None, None, C.byref(n)))
+        xyz = np.empty((n.value, 3), dtype=np.float64)
+        rgb = np.empty((n.value, 3), dtype=np.uint8)
+        extra = np.empty((n.value, *extra_shape), dtype=np.int32)
+        if n.value:
+            self._ck(call(n.value, _p(xyz), _p(rgb), _p(extra), C.byref(n)))
+        return xyz, rgb, extra
+
     def points(self, view):
         """The coloured point cloud of the view's depth map (sr_get_points): xyz (n, 3) float64, rgb (n, 3) uint8
         and the pixel index y * w + x (n,) int32 of every point, in row-major pixel order."""
-        n = C.c_int64(0)
-        self._ck(self._L.sr_get_points(self._h, int(view), 0, None, None, None, C.byref(n)))
-        xyz = np.empty((n.value, 3), dtype=np.float64)
-        rgb = np.empty((n.value, 3), dtype=np.uint8)
-        pixel = np.empty(n.value, dtype=np.int32)
-        if n.value:
-            self._ck(self._L.sr_get_points(self._h, int(view), n.value, _p(xyz), _p(rgb), _p(pixel), C.byref(n)))
-        return xyz, rgb, pixel
+        return self._count_then_fill(lambda *out: self._L.sr_get_points(self._h, int(view), *out), ())
 
     def fuse_points(self, max_dist, min_views=1):
         """One de-duplicated point cloud of all views' depth maps (sr_fuse_points): xyz (n, 3) float64, rgb (n, 3)
         uint8 and the source (view, y * w + x) (n, 2) int32 of every point, view-major, row-major within a view."""
-        n = C.c_int64(0)
-        self._ck(self._L.sr_fuse_points(self._h, float(max_dist), int(min_views), 0, None, None, None, C.byref(n)))
-        xyz = np.empty((n.value, 3), dtype=np.float64)
-        rgb = np.empty((n.value, 3), dtype=np.uint8)
-        source = np.empty((n.value, 2), dtype=np.int32)
-        if n.value:
-            self._ck(self._L.sr_fuse_points(self._h, float(max_dist), int(min_views), n.value, _p(xyz), _p(rgb),
-                                            _p(source), C.byref(n)))
-        return xyz, rgb, source
+        return self._count_then_fill(
+            lambda *out: self._L.sr_fuse_points(self._h, float(max_dist), int(min_views), *out), (2,))
 
     # -- building blocks -------------------------------------------------------------------
     def unproject_grid(self, view):

@@ -128,6 +128,8 @@ struct sr_ctx {
     int peaks_view = -1;
     void *d_scratch = nullptr;
     size_t scratch_cap = 0;
+    void *d_out = nullptr;  // variable-length results (point clouds), apart from the scratch that counts them
+    size_t out_cap = 0;
     int64_t launches = 0;
     size_t tap_budget = (size_t)8 << 30;
     unsigned long long *d_stats = nullptr;  // SR_MATCH_STATS=1: counters of the screened match kernel
@@ -243,6 +245,25 @@ int grow(sr_ctx *ctx, cudaStream_t st, T *&p, size_t &cap, size_t bytes) {
 
 int ensure_scratch(sr_ctx *ctx, size_t bytes) { return grow(ctx, ctx->stream, ctx->d_scratch, ctx->scratch_cap, bytes); }
 
+// Byte offsets of the pieces carved out of one buffer start on 256-byte boundaries.
+constexpr size_t align256(size_t bytes) { return (bytes + 255) / 256 * 256; }
+
+// Camera::unproject of the pixel centres of rows [row0, row0 + rows) into the [6][h][w] table `out`.
+int launch_rays(sr_ctx *ctx, const sr_camera &cam, int row0, int rows, double scale, double *out, cudaStream_t st) {
+    rays_kernel<<<(unsigned)(((size_t)rows * ctx->w + 127) / 128), 128, 0, st>>>(cam, ctx->w, ctx->h, row0, rows, scale, out);
+    CKL();
+    return SR_OK;
+}
+
+// The maps of a view read "not computed": NaN depth (twoviewstereo.cpp:118-119) and best cost, index NONE.
+int reset_maps(sr_ctx *ctx, ViewDev &v) {
+    const size_t n = (size_t)ctx->w * ctx->h;
+    CK(cudaMemsetAsync(v.depth, 0xff, n * 8, ctx->stream));
+    CK(cudaMemsetAsync(v.best, 0xff, n * 8, ctx->stream));
+    CK(cudaMemsetAsync(v.index, 0xff, n * 4, ctx->stream));
+    return SR_OK;
+}
+
 // Support weights (kind: SR_WEIGHT_*) of view v into W: of the pixels of rows [row0, row0 + rows), or, when
 // list_x is given, of the list_n window centres (list_x, list_y).
 int launch_weights(sr_ctx *ctx, const ViewDev &v, int kind, int radius, double *W, int row0, int rows, cudaStream_t st,
@@ -315,7 +336,13 @@ int join_lanes(sr_ctx *ctx) {
     std::fill(ctx->view_lane.begin(), ctx->view_lane.end(), -1);
     return SR_OK;
 }
-#define JOIN() CKR(join_lanes(ctx))
+
+// The preamble of every entry point that touches the device: select the context's device, then (join) order the
+// views still running on the lanes before the context stream.
+int enter(sr_ctx *ctx, bool join = true) {
+    CK(cudaSetDevice(ctx->device));
+    return join ? join_lanes(ctx) : SR_OK;
+}
 
 int check_view(sr_ctx *ctx, int v) {
     if (!ctx) return SR_ERR_INVALID;
@@ -324,10 +351,14 @@ int check_view(sr_ctx *ctx, int v) {
     return SR_OK;
 }
 
+int check_params(sr_ctx *ctx) {
+    return ctx->have_params ? SR_OK : fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+}
+
 // Arguments of sr_run_view / sr_run_view_curve; [r0, r1) is the row range to compute.
 int check_run(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn, int &r0, int &r1) {
     CKR(check_view(ctx, ref));
-    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    CKR(check_params(ctx));
     if (!nbrs || nn <= 0 || nn > SR_MAX_NBRS) return fail(ctx, SR_ERR_INVALID, "1..8 neighbour views required");
     for (int j = 0; j < nn; ++j)
         if (nbrs[j] < 0 || nbrs[j] >= ctx->V || nbrs[j] == ref) return fail(ctx, SR_ERR_INVALID, "bad neighbour index");
@@ -405,6 +436,81 @@ int run_match(sr_ctx *ctx, const MatchArgs &ma, cudaStream_t st) {
     return SR_OK;
 }
 
+// The fields the candidate builds of the reference view `ref` against neighbour `nbr` (BuildArgs, BuildRefrArgs,
+// CurveArgs) share, for rows [row0, row0 + rows) and the reference's ray table `rays`.
+template <typename A>
+void pair_fields(A &a, const sr_ctx *ctx, int ref, int nbr, const double *rays, int row0, int rows, bool mvs) {
+    a.nbr = ctx->cams[nbr];
+    memcpy(a.prin, ctx->cams[ref].prin_dir, sizeof(a.prin));
+    memcpy(a.C, ctx->cams[ref].C, sizeof(a.C));
+    a.rays = rays;
+    a.depth_table = ctx->d_depth_table;
+    a.ref_mask = ctx->views[ref].mask;
+    a.w = ctx->w;
+    a.h = ctx->h;
+    a.row0 = row0;
+    a.rows = rows;
+    a.D = ctx->params.num_levels;
+    a.mvs = mvs;
+}
+
+int d2h(sr_ctx *ctx, void *dst, const void *src, size_t bytes, int view = -1) {
+    // a view still on a lane: nothing on the context stream has touched its maps since (that would have joined
+    // the lanes), so its own event is all this copy has to wait for
+    const bool on_lane = view >= 0 && view < (int)ctx->view_lane.size() && ctx->view_lane[view] >= 0 &&
+                         view < (int)ctx->view_done.size() && ctx->view_done[view] && ctx->copy_stream;
+    CKR(enter(ctx, !on_lane));
+    if (on_lane) CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->view_done[view], 0));
+    cudaStream_t st = on_lane ? ctx->copy_stream : ctx->stream;
+    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return SR_OK;
+}
+
+// Downloads the device's [k][n] planes at src into the [n][k] layout the API documents.
+int d2h_transposed(sr_ctx *ctx, double *out, const double *src, size_t n, size_t k) {
+    if (!out) return fail(ctx, SR_ERR_INVALID, "the output array is null");
+    std::vector<double> planar(n * k);
+    CKR(d2h(ctx, planar.data(), src, n * k * sizeof(double)));
+    for (size_t i = 0; i < n; ++i)
+        for (size_t j = 0; j < k; ++j) out[i * k + j] = planar[j * n + i];
+    return SR_OK;
+}
+
+// Uploads the host's [n][k] layout at in as the device's [k][n] planes at dst.
+int h2d_transposed(sr_ctx *ctx, double *dst, const double *in, size_t n, size_t k) {
+    std::vector<double> planar(n * k);
+    for (size_t i = 0; i < n; ++i)
+        for (size_t j = 0; j < k; ++j) planar[j * n + i] = in[i * k + j];
+    CK(cudaMemcpyAsync(dst, planar.data(), n * k * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SR_OK;
+}
+
+// The second half of count-then-fill (sr_get_points, sr_fuse_points), once the counting kernels have left the
+// number of points at d_total.  *out_count receives it; a call with capacity 0, or without points, ends there.
+// Otherwise write(xyz, extra, rgb) fills the output buffer [xyz 3n doubles][extra n * extra_ints][rgb 3n]
+// (extra is null when out_extra is) and the arrays are downloaded.
+template <typename Write>
+int fill_points(sr_ctx *ctx, const long long *d_total, int64_t capacity, int64_t *out_count, const char *too_small,
+                double *out_xyz, uint8_t *out_rgb, int32_t *out_extra, int extra_ints, Write write) {
+    long long total = 0;
+    CKR(d2h(ctx, &total, d_total, sizeof(total)));
+    *out_count = total;
+    if (capacity == 0 || total == 0) return SR_OK;
+    if (capacity < total) return fail(ctx, SR_ERR_INVALID, too_small);
+    const size_t n = (size_t)total;
+    CKR(grow(ctx, ctx->stream, ctx->d_out, ctx->out_cap, n * (3 * sizeof(double) + extra_ints * sizeof(int32_t) + 3)));
+    double *xyz = (double *)ctx->d_out;
+    int32_t *extra = (int32_t *)(xyz + 3 * n);
+    uint8_t *rgb = (uint8_t *)(extra + extra_ints * n);
+    CKR(write(xyz, out_extra ? extra : nullptr, rgb));
+    CKR(d2h(ctx, out_xyz, xyz, n * 3 * sizeof(double)));
+    CKR(d2h(ctx, out_rgb, rgb, n * 3));
+    if (out_extra) CKR(d2h(ctx, out_extra, extra, n * extra_ints * sizeof(int32_t)));
+    return SR_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -475,6 +581,7 @@ void sr_ctx_destroy(sr_ctx *c) {
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     dfree(c->d_scratch);
+    dfree(c->d_out);
     cudaStreamDestroy(c->own_stream);
     delete c;
 }
@@ -488,10 +595,7 @@ void sr_clear_cancel(sr_ctx *c) {
 }
 int sr_set_stream(sr_ctx *c, void *s) {
     if (!c) return SR_ERR_INVALID;
-    {
-        sr_ctx *ctx = c;
-        JOIN();  // views still running on the lanes are ordered before whatever follows on the old stream
-    }
+    CKR(enter(c));  // views still running on the lanes are ordered before whatever follows on the old stream
     c->stream = s ? (cudaStream_t)s : c->own_stream;
     return SR_OK;
 }
@@ -524,8 +628,7 @@ int sr_set_views(sr_ctx *ctx, int V, const sr_camera *cams, const uint8_t *const
     if (!ctx) return SR_ERR_INVALID;
     if (V <= 0 || !cams || !rgba8 || w <= 0 || h <= 0 || w > 16384 || h > 16384)
         return fail(ctx, SR_ERR_INVALID, "sr_set_views: bad arguments (1 <= w,h <= 16384)");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     const size_t n = (size_t)w * h;
     if (V != ctx->V || w != ctx->w || h != ctx->h) {
         CK(cudaStreamSynchronize(ctx->stream));
@@ -571,9 +674,7 @@ int sr_set_views(sr_ctx *ctx, int V, const sr_camera *cams, const uint8_t *const
         // results: "not computed" (NaN depth, index NONE) under an all-WHITE mask, until a gather fills them.
         for (ViewDev &v : ctx->views) {
             CK(cudaMemsetAsync(v.mask, 255, n, ctx->stream));
-            CK(cudaMemsetAsync(v.depth, 0xff, n * 8, ctx->stream));
-            CK(cudaMemsetAsync(v.best, 0xff, n * 8, ctx->stream));
-            CK(cudaMemsetAsync(v.index, 0xff, n * 4, ctx->stream));
+            CKR(reset_maps(ctx, v));
         }
     }
     ctx->cams.assign(cams, cams + V);
@@ -590,10 +691,7 @@ int sr_set_views(sr_ctx *ctx, int V, const sr_camera *cams, const uint8_t *const
         prep_view_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(v.rgba, v.mask, w, h, v.gray_pix,
                                                                              v.gray_two, v.gray_msk, v.edges, v.gray_pix_f, screen_pitch(w));
         CKL();
-        // results start as "not computed": NaN depth (twoviewstereo.cpp:118-119), index NONE
-        CK(cudaMemsetAsync(v.depth, 0xff, n * 8, ctx->stream));
-        CK(cudaMemsetAsync(v.best, 0xff, n * 8, ctx->stream));
-        CK(cudaMemsetAsync(v.index, 0xff, n * 4, ctx->stream));
+        CKR(reset_maps(ctx, v));  // results start as "not computed"
     }
     return SR_OK;
 }
@@ -611,8 +709,7 @@ int sr_set_params(sr_ctx *ctx, const sr_params *p) {
     ctx->have_params = true;
     ctx->depth_table.resize(p->num_levels);
     for (int d = 0; d < p->num_levels; ++d) ctx->depth_table[d] = depth_from_label(*p, d);
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     CKR(grow(ctx, ctx->stream, ctx->d_depth_table, ctx->depth_table_cap, sizeof(double) * p->num_levels));
     CK(cudaMemcpyAsync(ctx->d_depth_table, ctx->depth_table.data(), sizeof(double) * p->num_levels,
                        cudaMemcpyHostToDevice, ctx->stream));
@@ -643,7 +740,6 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     int r0, r1;
     CKR(check_run(ctx, ref, nbrs, nn, r0, r1));
     const sr_params &P = ctx->params;
-    CK(cudaSetDevice(ctx->device));
     const int w = ctx->w, h = ctx->h, D = P.num_levels;
     const size_t n = (size_t)w * h;
     ViewDev &A = ctx->views[ref];
@@ -651,7 +747,7 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     // Where this view runs: one of the two lanes (its own stream and scratch), or the context stream when
     // something context-wide is written (kept volume, peak lists, statistics, per-stage timing).
     const bool on_lane = ctx->num_lanes > 1 && !ctx->profiling && !P.keep_cost_volume && !ctx->d_stats;
-    if (!on_lane) JOIN();
+    CKR(enter(ctx, !on_lane));
     sr_ctx::Lane *L = on_lane ? &ctx->lanes[ctx->next_lane] : nullptr;
     cudaStream_t st = on_lane ? L->stream : ctx->stream;
     Scratch &S = on_lane ? L->s : ctx->s;
@@ -668,8 +764,7 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     }
     CKR(grow(ctx, st, S.rays, S.rays_cap, n * 6 * 8));  // (the context's set has it from sr_set_views)
 
-    rays_kernel<<<(unsigned)(((size_t)(r1 - r0) * w + 127) / 128), 128, 0, st>>>(ctx->cams[ref], w, h, r0, r1 - r0, P.image_scale, S.rays);
-    CKL();
+    CKR(launch_rays(ctx, ctx->cams[ref], r0, r1 - r0, P.image_scale, S.rays, st));
 
     // Row bands bound the scratch (tap volume nn*D*rows*w*4 bytes + support weights
     // WN*rows*w*8 bytes); a kept cost volume needs one band.
@@ -703,22 +798,11 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
             if (nb.is_refractive && ctx->use_refr_build) {
                 // refractive target view: hoisted-affine reprojection + Newton on the quartic in x/r
                 BuildRefrArgs ra;
-                ra.nbr = nb;
+                pair_fields(ra, ctx, ref, nbrs[j], S.rays, b0, rows, mvs);
                 refr_pixel_map(nb, mvs ? 0.0 : -0.5, P.image_scale, ra.Kn, ra.fxs, ra.cxs, ra.fys, ra.cys);
-                memcpy(ra.prin, ctx->cams[ref].prin_dir, sizeof(ra.prin));
-                memcpy(ra.C, ctx->cams[ref].C, sizeof(ra.C));
-                ra.rays = S.rays;
-                ra.depth_table = ctx->d_depth_table;
-                ra.ref_mask = A.mask;
                 ra.nbr_mask = ctx->views[nbrs[j]].all_white ? nullptr : ctx->views[nbrs[j]].mask;
                 ra.taps = S.taps + (size_t)j * D * plane;
-                ra.w = w;
-                ra.h = h;
-                ra.row0 = b0;
-                ra.rows = rows;
-                ra.D = D;
                 ra.d_chunk = REFR_CHUNK;
-                ra.mvs = mvs;
                 ra.check = ctx->d_stats ? ctx->d_stats + 8 : nullptr;
                 const dim3 grid(gx, (D + ra.d_chunk - 1) / ra.d_chunk);
                 if (!mvs) build_refr_kernel<false, false><<<grid, 128, 0, st>>>(ra);
@@ -728,22 +812,11 @@ int sr_run_view(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
                 continue;
             }
             BuildArgs ba;
-            ba.nbr = nb;
-            memcpy(ba.prin, ctx->cams[ref].prin_dir, sizeof(ba.prin));
-            memcpy(ba.C, ctx->cams[ref].C, sizeof(ba.C));
-            ba.rays = S.rays;
-            ba.depth_table = ctx->d_depth_table;
-            ba.ref_mask = A.mask;
+            pair_fields(ba, ctx, ref, nbrs[j], S.rays, b0, rows, mvs);
             ba.nbr_mask = ctx->views[nbrs[j]].mask;
             ba.taps = S.taps + (size_t)j * D * plane;
-            ba.w = w;
-            ba.h = h;
-            ba.row0 = b0;
-            ba.rows = rows;
-            ba.D = D;
             ba.d_chunk = d_chunk;
             ba.scale = P.image_scale;
-            ba.mvs = mvs;
             build_kernel<<<dim3(gx, (D + d_chunk - 1) / d_chunk), 128, 0, st>>>(ba);
             CKL();
         }
@@ -778,8 +851,7 @@ int sr_set_profiling(sr_ctx *ctx, int on) {
 // call), out[2] = number of build launches' bands, out[3] = number of match launches.
 int sr_get_stage_ms(sr_ctx *ctx, double *out4) {
     if (!ctx || !out4) return SR_ERR_INVALID;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     CK(cudaStreamSynchronize(ctx->stream));
     out4[0] = out4[1] = out4[2] = out4[3] = 0;
     for (size_t i = 0; i + 2 < ctx->prof_events.size(); i += 3) {
@@ -799,7 +871,7 @@ int sr_get_stage_ms(sr_ctx *ctx, double *out4) {
 int sr_get_build_stats(sr_ctx *ctx, uint64_t *out4) {
     if (!ctx || !out4) return SR_ERR_INVALID;
     if (!ctx->d_stats) return fail(ctx, SR_ERR_STATE, "build statistics are off (set SR_MATCH_STATS=1 before sr_ctx_create)");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, false));
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaMemcpy(out4, ctx->d_stats + 8, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     return SR_OK;
@@ -811,7 +883,7 @@ int sr_get_build_stats(sr_ctx *ctx, uint64_t *out4) {
 int sr_get_match_stats(sr_ctx *ctx, uint64_t *out8) {
     if (!ctx || !out8) return SR_ERR_INVALID;
     if (!ctx->d_stats) return fail(ctx, SR_ERR_STATE, "match statistics are off (set SR_MATCH_STATS=1 before sr_ctx_create)");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, false));
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaMemcpy(out8, ctx->d_stats, 8 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     return SR_OK;
@@ -823,8 +895,7 @@ static int ensure_rays(sr_ctx *ctx, int v) {
     const double scale = ctx->params.image_scale;
     if (!d.rays) CK(cudaMalloc(&d.rays, n * 6 * 8));
     if (d.rays_scale != scale) {
-        rays_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(ctx->cams[v], ctx->w, ctx->h, 0, ctx->h, scale, d.rays);
-        CKL();
+        CKR(launch_rays(ctx, ctx->cams[v], 0, ctx->h, scale, d.rays, ctx->stream));
         d.rays_scale = scale;
     }
     return SR_OK;
@@ -839,11 +910,10 @@ int sr_run_view_curve(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     const bool mvs = (P.select_kind == SR_SELECT_MVS);
     if (P.keep_cost_volume & 1) return fail(ctx, SR_ERR_INVALID, "curve mode keeps no cost volume (candidates are not labels)");
     if (mvs && P.cost_kind != SR_COST_NCC_MVS) return fail(ctx, SR_ERR_INVALID, "multi-view curve search uses SR_COST_NCC_MVS");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     cudaStream_t st = ctx->stream;
     Scratch &S = ctx->s;
-    const int w = ctx->w, h = ctx->h, D = P.num_levels;
+    const int w = ctx->w, D = P.num_levels;
     ViewDev &A = ctx->views[ref];
     CKR(ensure_rays(ctx, ref));
     for (int j = 0; j < nn; ++j) CKR(ensure_rays(ctx, nbrs[j]));
@@ -852,24 +922,12 @@ int sr_run_view_curve(sr_ctx *ctx, int ref, const int32_t *nbrs, int nn) {
     const size_t per_row_w = wn * w * 8;
 
     auto curve_args = [&](int j, int b0, int rows) {
-        const sr_camera &nb = ctx->cams[nbrs[j]];
         CurveArgs ca;
         memset(&ca, 0, sizeof(ca));
-        ca.nbr = nb;
-        refr_pixel_map(nb, 0.0, P.image_scale, ca.Kn, ca.fxs, ca.cxs, ca.fys, ca.cys);
-        memcpy(ca.prin, ctx->cams[ref].prin_dir, sizeof(ca.prin));
-        memcpy(ca.C, ctx->cams[ref].C, sizeof(ca.C));
+        pair_fields(ca, ctx, ref, nbrs[j], A.rays, b0, rows, mvs);
+        refr_pixel_map(ca.nbr, 0.0, P.image_scale, ca.Kn, ca.fxs, ca.cxs, ca.fys, ca.cys);
         ca.scale = P.image_scale;
-        ca.rays = A.rays;
-        ca.depth_table = ctx->d_depth_table;
-        ca.ref_mask = A.mask;
         ca.nbr_mask = ctx->views[nbrs[j]].mask;
-        ca.w = w;
-        ca.h = h;
-        ca.row0 = b0;
-        ca.rows = rows;
-        ca.D = D;
-        ca.mvs = mvs;
         return ca;
     };
     auto launch_curve = [&](const CurveArgs &ca, unsigned gx, bool masked) {
@@ -968,8 +1026,7 @@ int sr_cross_check(sr_ctx *ctx, int two_view, double threshold) {
     if (!ctx) return SR_ERR_INVALID;
     if (ctx->V == 0 || !ctx->have_params) return fail(ctx, SR_ERR_STATE, "views/params not set");
     if (two_view && ctx->V != 2) return fail(ctx, SR_ERR_INVALID, "two-view cross-check needs exactly 2 views");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     const size_t n = (size_t)ctx->w * ctx->h;
     // View by view, in place, in index order: view v sees the already-updated maps of views < v,
     // exactly as twoviewstereo.cpp:604-670 / multiviewstereo.cpp:427-431 do.
@@ -993,48 +1050,25 @@ int sr_cross_check(sr_ctx *ctx, int two_view, double threshold) {
 
 int sr_flush(sr_ctx *ctx) {
     if (!ctx) return SR_ERR_INVALID;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
-    return SR_OK;
+    return enter(ctx);
 }
 int sr_synchronize(sr_ctx *ctx) {
     if (!ctx) return SR_ERR_INVALID;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
-    CK(cudaStreamSynchronize(ctx->stream));
-    return SR_OK;
-}
-
-static int d2h(sr_ctx *ctx, void *dst, const void *src, size_t bytes, int view = -1) {
-    CK(cudaSetDevice(ctx->device));
-    if (view >= 0 && view < (int)ctx->view_lane.size() && ctx->view_lane[view] >= 0 && view < (int)ctx->view_done.size() &&
-        ctx->view_done[view] && ctx->copy_stream) {
-        // the view is still on a lane: nothing on the context stream has touched its maps since (that would
-        // have joined the lanes), so its own event is all this copy has to wait for
-        CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->view_done[view], 0));
-        CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->copy_stream));
-        CK(cudaStreamSynchronize(ctx->copy_stream));
-        return SR_OK;
-    }
-    JOIN();
-    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CKR(enter(ctx));
     CK(cudaStreamSynchronize(ctx->stream));
     return SR_OK;
 }
 
 int sr_get_depth_index(sr_ctx *ctx, int view, int32_t *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     return d2h(ctx, out, ctx->views[view].index, (size_t)ctx->w * ctx->h * 4, view);
 }
 int sr_get_depth(sr_ctx *ctx, int view, double *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     return d2h(ctx, out, ctx->views[view].depth, (size_t)ctx->w * ctx->h * 8, view);
 }
 int sr_get_best_cost(sr_ctx *ctx, int view, double *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     return d2h(ctx, out, ctx->views[view].best, (size_t)ctx->w * ctx->h * 8, view);
 }
 int sr_get_cost_volume(sr_ctx *ctx, float *out, size_t out_elems) {
@@ -1044,37 +1078,25 @@ int sr_get_cost_volume(sr_ctx *ctx, float *out, size_t out_elems) {
     return d2h(ctx, out, ctx->d_volume, ctx->vol_elems * 4);
 }
 int sr_get_peaks(sr_ctx *ctx, int view, double *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     if (!out) return SR_ERR_INVALID;
     if (ctx->peaks_view != view) return fail(ctx, SR_ERR_STATE, "no peak lists kept for this view (set keep_cost_volume |= 2 and run it)");
-    const size_t n = (size_t)ctx->w * ctx->h;
-    std::vector<double> planar(n * 18);
-    rc = d2h(ctx, planar.data(), ctx->d_peaks, n * 18 * 8);
-    if (rc) return rc;
-    for (size_t i = 0; i < n; ++i)  // device layout [9][2][pixel] -> the [pixel][9][2] the API documents
-        for (int k = 0; k < 18; ++k) out[i * 18 + k] = planar[(size_t)k * n + i];
-    return SR_OK;
+    return d2h_transposed(ctx, out, ctx->d_peaks, (size_t)ctx->w * ctx->h, 18);  // [9][2][pixel] -> [pixel][9][2]
 }
 int sr_set_depth(sr_ctx *ctx, int view, const double *depth) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(check_view(ctx, view));
+    CKR(enter(ctx));
     CK(cudaMemcpyAsync(ctx->views[view].depth, depth, (size_t)ctx->w * ctx->h * 8, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return SR_OK;
 }
 int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
-    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    CKR(check_view(ctx, view));
+    CKR(check_params(ctx));
     if (!mvs) return fail(ctx, SR_ERR_INVALID, "two-view HSV depth image is produced by the host class (QColor semantics)");
+    CKR(enter(ctx));  // the view may still be running on a lane
     const size_t n = (size_t)ctx->w * ctx->h;
-    rc = ensure_scratch(ctx, n * 4);
-    if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();  // the view may still be running on a lane
+    CKR(ensure_scratch(ctx, n * 4));
     depth_image_mvs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(
         ctx->views[view].depth, ctx->views[view].mask, (int)n, ctx->params.min_depth, ctx->params.max_depth,
         (uchar4 *)ctx->d_scratch);
@@ -1084,14 +1106,12 @@ int sr_get_depth_image(sr_ctx *ctx, int view, int mvs, uint8_t *out) {
 
 int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint8_t *out_rgb, int32_t *out_pixel,
                   int64_t *out_count) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     if (!out_count || capacity < 0 || (capacity > 0 && (!out_xyz || !out_rgb)))
         return fail(ctx, SR_ERR_INVALID, "sr_get_points: out_count, and out_xyz and out_rgb when capacity > 0, are required");
-    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    CKR(check_params(ctx));
     if (!ctx->views[view].have_image) return fail(ctx, SR_ERR_STATE, "the view was given no image in sr_set_views");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();  // the view may still be running on a lane
+    CKR(enter(ctx));  // the view may still be running on a lane
     const int h = ctx->h;
     PointsArgs pa;
     memset(&pa, 0, sizeof(pa));
@@ -1102,37 +1122,22 @@ int sr_get_points(sr_ctx *ctx, int view, int64_t capacity, double *out_xyz, uint
     pa.h = h;
     pa.scale = ctx->params.image_scale;
     pa.min_depth = ctx->params.min_depth;
-    // scratch: [row offsets][xyz][pixel][rgb]
-    const size_t off_bytes = ((size_t)(h + 1) * sizeof(long long) + 255) / 256 * 256;
-    auto count_points = [&]() -> int {
-        pa.offsets = (long long *)ctx->d_scratch;
-        points_count_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
-        CKL();
-        points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(pa.offsets, h);
-        CKL();
-        return SR_OK;
-    };
-    CKR(ensure_scratch(ctx, off_bytes));
-    CKR(count_points());
-    long long total = 0;
-    CKR(d2h(ctx, &total, pa.offsets + h, sizeof(total)));
-    *out_count = total;
-    if (capacity == 0 || total == 0) return SR_OK;
-    if (capacity < total) return fail(ctx, SR_ERR_INVALID, "sr_get_points: capacity is smaller than the number of points");
-    const size_t n = (size_t)total;
-    const size_t cap0 = ctx->scratch_cap;
-    CKR(ensure_scratch(ctx, off_bytes + n * (3 * sizeof(double) + sizeof(int32_t) + 3)));
-    if (ctx->scratch_cap != cap0) CKR(count_points());  // a new buffer: the offsets went with the old one
-    pa.xyz = (double *)((char *)ctx->d_scratch + off_bytes);
-    int32_t *d_pixel = (int32_t *)(pa.xyz + 3 * n);
-    pa.pixel = out_pixel ? d_pixel : nullptr;
-    pa.rgb = (uint8_t *)(d_pixel + n);
-    points_write_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
+    // scratch: the row offsets; the points go to the output buffer
+    CKR(ensure_scratch(ctx, (size_t)(h + 1) * sizeof(long long)));
+    pa.offsets = (long long *)ctx->d_scratch;
+    points_count_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
     CKL();
-    CKR(d2h(ctx, out_xyz, pa.xyz, n * 3 * sizeof(double)));
-    CKR(d2h(ctx, out_rgb, pa.rgb, n * 3));
-    if (out_pixel) CKR(d2h(ctx, out_pixel, d_pixel, n * sizeof(int32_t)));
-    return SR_OK;
+    points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(pa.offsets, h);
+    CKL();
+    return fill_points(ctx, pa.offsets + h, capacity, out_count, "sr_get_points: capacity is smaller than the number of points",
+                       out_xyz, out_rgb, out_pixel, 1, [&](double *xyz, int32_t *pixel, uint8_t *rgb) -> int {
+                           pa.xyz = xyz;
+                           pa.pixel = pixel;
+                           pa.rgb = rgb;
+                           points_write_kernel<<<h, POINTS_THREADS, 0, ctx->stream>>>(pa);
+                           CKL();
+                           return SR_OK;
+                       });
 }
 
 int sr_fuse_points(sr_ctx *ctx, double max_dist, int min_views, int64_t capacity, double *out_xyz, uint8_t *out_rgb,
@@ -1143,14 +1148,12 @@ int sr_fuse_points(sr_ctx *ctx, double max_dist, int min_views, int64_t capacity
     if (!(max_dist >= 0.0 && std::isfinite(max_dist)) || min_views < 0)
         return fail(ctx, SR_ERR_INVALID, "sr_fuse_points: max_dist must be finite and >= 0, min_views >= 0");
     if (ctx->V == 0) return fail(ctx, SR_ERR_STATE, "sr_set_views has not been called");
-    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    CKR(check_params(ctx));
     for (const ViewDev &v : ctx->views)
         if (!v.have_image) return fail(ctx, SR_ERR_STATE, "sr_fuse_points: a view was given no image in sr_set_views");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();  // a view may still be running on a lane
+    CKR(enter(ctx));  // a view may still be running on a lane
     const int rows = ctx->V * ctx->h;
     const size_t N = (size_t)ctx->V * ctx->w * ctx->h;
-    auto align = [](size_t b) { return (b + 255) / 256 * 256; };
     FuseArgs fa;
     memset(&fa, 0, sizeof(fa));
     fa.cams = ctx->d_cams;
@@ -1163,44 +1166,29 @@ int sr_fuse_points(sr_ctx *ctx, double max_dist, int min_views, int64_t capacity
     fa.min_depth = ctx->params.min_depth;
     fa.max_dist = max_dist;
     fa.min_views = min_views;
-    // scratch: [row offsets][fused xyz planes][support][rgbe], then the points' [xyz][source][rgb]
-    const size_t off_bytes = align((size_t)(rows + 1) * sizeof(long long));
-    const size_t pix_bytes = off_bytes + N * (3 * sizeof(double) + sizeof(int32_t) + sizeof(uint32_t));
-    auto count_points = [&]() -> int {
-        char *base = (char *)ctx->d_scratch;
-        fa.offsets = (long long *)base;
-        fa.fxyz = (double *)(base + off_bytes);
-        fa.support = (int32_t *)(fa.fxyz + 3 * N);
-        fa.rgbe = (uint32_t *)(fa.support + N);
-        fuse_support_kernel<<<(unsigned)((N + FUSE_THREADS - 1) / FUSE_THREADS), FUSE_THREADS, 0, ctx->stream>>>(fa);
-        CKL();
-        fuse_emit_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
-        CKL();
-        points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(fa.offsets, rows);
-        CKL();
-        return SR_OK;
-    };
-    CKR(ensure_scratch(ctx, pix_bytes));
-    CKR(count_points());
-    long long total = 0;
-    CKR(d2h(ctx, &total, fa.offsets + rows, sizeof(total)));
-    *out_count = total;
-    if (capacity == 0 || total == 0) return SR_OK;
-    if (capacity < total) return fail(ctx, SR_ERR_INVALID, "sr_fuse_points: capacity is smaller than the number of points");
-    const size_t n = (size_t)total;
-    const size_t cap0 = ctx->scratch_cap;
-    CKR(ensure_scratch(ctx, pix_bytes + n * (3 * sizeof(double) + 2 * sizeof(int32_t) + 3)));
-    if (ctx->scratch_cap != cap0) CKR(count_points());  // a new buffer: the scratch went with the old one
-    fa.xyz = (double *)((char *)ctx->d_scratch + pix_bytes);
-    int32_t *d_source = (int32_t *)(fa.xyz + 3 * n);
-    fa.source = out_source ? d_source : nullptr;
-    fa.rgb = (uint8_t *)(d_source + 2 * n);
-    fuse_write_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
+    // scratch: [row offsets][fused xyz planes][support][rgbe]; the points go to the output buffer
+    const size_t off_bytes = align256((size_t)(rows + 1) * sizeof(long long));
+    CKR(ensure_scratch(ctx, off_bytes + N * (3 * sizeof(double) + sizeof(int32_t) + sizeof(uint32_t))));
+    char *base = (char *)ctx->d_scratch;
+    fa.offsets = (long long *)base;
+    fa.fxyz = (double *)(base + off_bytes);
+    fa.support = (int32_t *)(fa.fxyz + 3 * N);
+    fa.rgbe = (uint32_t *)(fa.support + N);
+    fuse_support_kernel<<<(unsigned)((N + FUSE_THREADS - 1) / FUSE_THREADS), FUSE_THREADS, 0, ctx->stream>>>(fa);
     CKL();
-    CKR(d2h(ctx, out_xyz, fa.xyz, n * 3 * sizeof(double)));
-    CKR(d2h(ctx, out_rgb, fa.rgb, n * 3));
-    if (out_source) CKR(d2h(ctx, out_source, d_source, n * 2 * sizeof(int32_t)));
-    return SR_OK;
+    fuse_emit_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
+    CKL();
+    points_scan_kernel<<<1, POINTS_SCAN_THREADS, 0, ctx->stream>>>(fa.offsets, rows);
+    CKL();
+    return fill_points(ctx, fa.offsets + rows, capacity, out_count, "sr_fuse_points: capacity is smaller than the number of points",
+                       out_xyz, out_rgb, out_source, 2, [&](double *xyz, int32_t *source, uint8_t *rgb) -> int {
+                           fa.xyz = xyz;
+                           fa.source = source;
+                           fa.rgb = rgb;
+                           fuse_write_kernel<<<rows, POINTS_THREADS, 0, ctx->stream>>>(fa);
+                           CKL();
+                           return SR_OK;
+                       });
 }
 
 void sr_mrf_params_default(sr_mrf_params *p) {
@@ -1216,15 +1204,10 @@ int sr_set_peaks(sr_ctx *ctx, int view, const double *peaks) {
     CKR(check_view(ctx, view));
     if (!peaks) return fail(ctx, SR_ERR_INVALID, "sr_set_peaks: peaks is null");
     const size_t n = (size_t)ctx->w * ctx->h;
-    std::vector<double> planar(n * 18);
-    for (size_t i = 0; i < n; ++i)  // [pixel][9][2] -> the device's [9][2][pixel]
-        for (int k = 0; k < 18; ++k) planar[(size_t)k * n + i] = peaks[i * 18 + k];
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     ctx->peaks_view = -1;
     CKR(grow(ctx, ctx->stream, ctx->d_peaks, ctx->peaks_cap, n * 18 * 8));
-    CK(cudaMemcpyAsync(ctx->d_peaks, planar.data(), n * 18 * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+    CKR(h2d_transposed(ctx, ctx->d_peaks, peaks, n, 18));  // [pixel][9][2] -> the device's [9][2][pixel]
     ctx->peaks_view = view;
     return SR_OK;
 }
@@ -1239,7 +1222,7 @@ static bool mrf_term(double v, double cap, float &out) {
 int sr_mrf_select(sr_ctx *ctx, int view, const sr_mrf_params *mp, double *out_energy) {
     CKR(check_view(ctx, view));
     if (!mp) return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: params is null");
-    if (!ctx->have_params) return fail(ctx, SR_ERR_STATE, "sr_set_params has not been called");
+    CKR(check_params(ctx));
     if (ctx->peaks_view != view)
         return fail(ctx, SR_ERR_STATE, "no peak lists for this view (run it with keep_cost_volume |= 2, or sr_set_peaks)");
     const sr_params &P = ctx->params;
@@ -1259,14 +1242,12 @@ int sr_mrf_select(sr_ctx *ctx, int view, const sr_mrf_params *mp, double *out_en
         !(mp->smooth_weight * mp->smooth_trunc <= cap))
             return fail(ctx, SR_ERR_INVALID, "sr_mrf_select: iterations must be >= 0 and every term finite, >= 0 and at most "
                                          "1e30 (smooth_weight * smooth_trunc too)");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     const size_t n = (size_t)w * h;
     const unsigned blocks = (unsigned)((n + 255) / 256);
-    auto align = [](size_t b) { return (b + 255) / 256 * 256; };
     // scratch: [messages 4*10*n][unary 9*n][z 9*n] floats, [labels n], [energy partials][energy]
     const size_t msg_bytes = (size_t)4 * MRF_L * n * sizeof(float), slot_bytes = (size_t)MRF_K * n * sizeof(float);
-    const size_t lab_off = msg_bytes + 2 * slot_bytes, part_off = lab_off + align(n);
+    const size_t lab_off = msg_bytes + 2 * slot_bytes, part_off = lab_off + align256(n);
     CKR(ensure_scratch(ctx, part_off + ((size_t)blocks + 1) * sizeof(double)));
     char *base = (char *)ctx->d_scratch;
     ViewDev &V = ctx->views[view];
@@ -1302,29 +1283,18 @@ int sr_mrf_select(sr_ctx *ctx, int view, const sr_mrf_params *mp, double *out_en
 }
 
 int sr_unproject_grid(sr_ctx *ctx, int view, double *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
-    const size_t n = (size_t)ctx->w * ctx->h;
+    CKR(check_view(ctx, view));
+    CKR(enter(ctx));
     const double scale = ctx->have_params ? ctx->params.image_scale : 1.0;
-    rays_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(ctx->cams[view], ctx->w, ctx->h, 0, ctx->h, scale, ctx->s.rays);
-    CKL();
-    std::vector<double> soa(n * 6);
-    rc = d2h(ctx, soa.data(), ctx->s.rays, n * 6 * 8);
-    if (rc) return rc;
-    for (size_t i = 0; i < n; ++i)  // SoA (device layout) -> the (h,w,6) AoS the API documents
-        for (int k = 0; k < 6; ++k) out[i * 6 + k] = soa[k * n + i];
-    return SR_OK;
+    CKR(launch_rays(ctx, ctx->cams[view], 0, ctx->h, scale, ctx->s.rays, ctx->stream));
+    return d2h_transposed(ctx, out, ctx->s.rays, (size_t)ctx->w * ctx->h, 6);  // [6][h][w] -> [h][w][6]
 }
 
 int sr_project_points(sr_ctx *ctx, int view, int n, const double *xyz, double *out_xy, int32_t *out_ok) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     if (n <= 0) return SR_OK;
-    CK(cudaSetDevice(ctx->device));
-    rc = ensure_scratch(ctx, (size_t)n * (24 + 16 + 4));
-    if (rc) return rc;
+    CKR(enter(ctx, false));
+    CKR(ensure_scratch(ctx, (size_t)n * (24 + 16 + 4)));
     double *dx = (double *)ctx->d_scratch;
     double *dxy = dx + (size_t)3 * n;
     int32_t *dok = (int32_t *)(dxy + (size_t)2 * n);
@@ -1339,26 +1309,19 @@ int sr_project_points(sr_ctx *ctx, int view, int n, const double *xyz, double *o
 
 int sr_compute_weights(sr_ctx *ctx, int view, int kind, int radius, int n, const int32_t *cx, const int32_t *cy,
                        double *out) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     if (n <= 0) return SR_OK;
     if (radius < 1 || radius > 64 || kind < 0 || kind > 1) return fail(ctx, SR_ERR_INVALID, "bad radius/kind");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, false));
     const size_t wn = (size_t)(2 * radius + 1) * (2 * radius + 1);
-    rc = ensure_scratch(ctx, (size_t)n * 8 + (size_t)n * wn * 8);
-    if (rc) return rc;
+    CKR(ensure_scratch(ctx, (size_t)n * 8 + (size_t)n * wn * 8));
     int32_t *dcx = (int32_t *)ctx->d_scratch;
     int32_t *dcy = dcx + n;
     double *dW = (double *)(dcy + n);
     CK(cudaMemcpyAsync(dcx, cx, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(dcy, cy, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
     CKR(launch_weights(ctx, ctx->views[view], kind, radius, dW, 0, 0, ctx->stream, dcx, dcy, n));
-    std::vector<double> tmp((size_t)n * wn);
-    rc = d2h(ctx, tmp.data(), dW, (size_t)n * wn * 8);
-    if (rc) return rc;
-    for (int i = 0; i < n; ++i)  // device layout [tap][centre] -> the [centre][row][col] the API documents
-        for (size_t k = 0; k < wn; ++k) out[(size_t)i * wn + k] = tmp[k * n + i];
-    return SR_OK;
+    return d2h_transposed(ctx, out, dW, (size_t)n, wn);  // [tap][centre] -> [centre][row][col]
 }
 
 int sr_calibration_residuals_batch(sr_ctx *ctx, int num_models, int num_cams, const sr_camera *cams, int n,
@@ -1369,11 +1332,10 @@ int sr_calibration_residuals_batch(sr_ctx *ctx, int num_models, int num_cams, co
     if (n == 0) return SR_OK;
     for (int i = 0; i < 2 * n; ++i)
         if (view_pairs[i] < 0 || view_pairs[i] >= num_cams) return fail(ctx, SR_ERR_INVALID, "camera index out of range");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, false));
     const size_t ncam = (size_t)num_models * num_cams;
-    const size_t cam_bytes = ((sizeof(sr_camera) * ncam + 15) / 16) * 16;
-    int rc = ensure_scratch(ctx, cam_bytes + (size_t)n * (32 + 8) + (size_t)num_models * n * 8);
-    if (rc) return rc;
+    const size_t cam_bytes = align256(sizeof(sr_camera) * ncam);
+    CKR(ensure_scratch(ctx, cam_bytes + (size_t)n * (32 + 8) + (size_t)num_models * n * 8));
     char *base = (char *)ctx->d_scratch;
     sr_camera *dc = (sr_camera *)base;
     double *dpix = (double *)(base + cam_bytes);
@@ -1408,7 +1370,7 @@ int sr_comm_init(sr_ctx *ctx, const void *uid128, int rank, int nranks) {
     if (!ctx || !uid128 || nranks < 1 || rank < 0 || rank >= nranks) return SR_ERR_INVALID;
     std::string err;
     if (!load_nccl(err)) return fail(ctx, SR_ERR_NCCL, err);
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, false));
     Uid128 id;
     memcpy(id.b, uid128, 128);
     int r = g_nccl.CommInitRank(&ctx->comm, nranks, id, rank);
@@ -1433,8 +1395,7 @@ int sr_comm_allgather_views(sr_ctx *ctx, const int32_t *owner) {
     if (!ctx->comm) return fail(ctx, SR_ERR_STATE, "sr_comm_init has not been called");
     for (int v = 0; v < ctx->V; ++v)
         if (owner[v] < 0 || owner[v] >= ctx->nranks) return fail(ctx, SR_ERR_INVALID, "sr_comm_allgather_views: owner rank out of range");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     const size_t n = (size_t)ctx->w * ctx->h;
     int r = g_nccl.GroupStart();
     for (int v = 0; v < ctx->V && r == 0; ++v) r = bcast_maps(ctx, ctx->views[v], 0, n, owner[v]);
@@ -1445,15 +1406,13 @@ int sr_comm_allgather_views(sr_ctx *ctx, const int32_t *owner) {
 }
 
 int sr_comm_allgather_rows(sr_ctx *ctx, int view, const int32_t *row_begin, const int32_t *row_end) {
-    int rc = check_view(ctx, view);
-    if (rc) return rc;
+    CKR(check_view(ctx, view));
     if (!ctx->comm) return fail(ctx, SR_ERR_STATE, "sr_comm_init has not been called");
     if (!row_begin || !row_end) return fail(ctx, SR_ERR_INVALID, "sr_comm_allgather_rows: null row ranges");
     for (int k = 0; k < ctx->nranks; ++k)
         if (row_begin[k] < 0 || row_begin[k] > row_end[k] || row_end[k] > ctx->h)
             return fail(ctx, SR_ERR_INVALID, "sr_comm_allgather_rows: need 0 <= row_begin <= row_end <= height for every rank");
-    CK(cudaSetDevice(ctx->device));
-    JOIN();
+    CKR(enter(ctx));
     ViewDev &d = ctx->views[view];
     int r = g_nccl.GroupStart();
     for (int k = 0; k < ctx->nranks && r == 0; ++k) {

@@ -148,6 +148,21 @@ def test_bad_arguments_fail_loudly(ctx):
             run(0, [1, 2])  # two-view selection takes exactly one neighbour
 
 
+def test_null_outputs_are_invalid(ctx):
+    """A NULL output array of the transposing downloads is SR_ERR_INVALID with a message, not a host crash."""
+    SR_ERR_INVALID = 1  # include/sr_b200.h
+    cams, imgs, _, _ = refractive_arc_scene(V=3, w=32, h=24, masks=False)
+    ctx.set_views(cams, imgs, None)
+    assert ctx._L.sr_unproject_grid(ctx._h, 0, None) == SR_ERR_INVALID
+    assert b"null" in ctx._L.sr_last_error(ctx._h)
+    cx = np.array([5, 10], np.int32)
+    cy = np.array([6, 12], np.int32)
+    rc = ctx._L.sr_compute_weights(ctx._h, 0, 0, 2, cx.size, capi._p(cx), capi._p(cy), None)
+    assert rc == SR_ERR_INVALID
+    assert ctx.unproject_grid(0).shape == (24, 32, 6)  # the context is still usable
+    assert ctx.weights(0, 0, 2, cx, cy).shape == (2, 5, 5)
+
+
 def test_camera_only_views(ctx):
     """rgba8[i] == NULL: a view this context only needs the camera of (another rank computes it)."""
     cams, imgs, ms, _ = refractive_arc_scene(V=5, w=64, h=40, masks=False)
